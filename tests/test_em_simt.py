@@ -18,7 +18,8 @@ from gbrs_b200 import synth
 from gbrs_b200.quantify import hapmask_bytes
 from oracle import em_oracle as eo
 from tests import helpers as hp
-from tests import simt_em
+from tests import layouts, simt_em
+from tests import xref as xr
 
 pytestmark = pytest.mark.skipif(shutil.which("g++") is None, reason="g++ is needed to build the SIMT emulation")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -76,29 +77,65 @@ def test_emulated_wide_classes_short_items_and_alignment_counts():
 def test_emulated_column_pass_size_classes():
     """Every kind of column-pass work in one problem -- long items (a whole warp), short items of more than two quads
     (eight lanes), of two quads (two lanes, sixteen per warp) and of one quad (one lane, thirty-two per warp), partial and
-    full -- at the default item length; the trailer of item_desc agrees with the descriptors; updates of models 4 and 3
-    against the oracle."""
-    d = synth.generate(T=60, N=5000, H=8, sample_index=21)
+    full -- at the default item length, on a constructed layout (tests/layouts.py) so that all seven slot segments hold
+    items; the trailer of item_desc agrees with the descriptors; updates of models 4 and 3 against the extended-precision
+    reference, element-wise."""
+    d = layouts.make_layout(8, 64)
     gene_of = eo.gene_index(d.T, d.groups())
     pat = simt_em.HostPattern(synth.to_apm(d), gene_of=gene_of)
+    layouts.assert_layout_covers(pat.packed)
     n_items, nl = pat.info["n_items"], pat.info["n_long_items"]
     desc = pat.packed.arrays["item_desc"].reshape(-1, 4).astype(np.int64)
     assert desc.shape[0] == n_items + 2
     tr, desc = desc[n_items:].ravel(), desc[:n_items]
     lens = desc[:, 1] - desc[:, 0]
     p8, p4, f0, f8, f4 = (int(x) for x in tr[:5])
-    assert nl > 0 and nl < p8 < p4 < f0 <= f8 <= f4 <= n_items  # all partial size classes are present
-    assert np.all(lens[nl:p8] > 8) and np.all((lens[p8:p4] > 4) & (lens[p8:p4] <= 8)) and np.all(lens[p4:f0] <= 4)
+    assert 0 < nl < p8 < p4 < f0 < f8 < f4 < n_items  # every segment holds items
+    assert np.all(lens[:nl] > 64) and np.all(lens[nl:p8] > 8) and np.all(lens[f0:f8] > 8)
+    assert np.all((lens[p8:p4] > 4) & (lens[p8:p4] <= 8)) and np.all(lens[p4:f0] <= 4)
+    assert np.all((lens[f8:f4] > 4) & (lens[f8:f4] <= 8)) and np.all(lens[f4:] <= 4)
     assert not desc[nl:f0, 3].any() and desc[f0:, 3].all()
+    x = xr.XRef(d, gene_of)
     eff = eo.effective_length_table(d.lengths)
     theta = pat.prepare(eff)
-    oapm = eo.apm_from_pairs(d.T, d.H, d.N, d.pair_class, d.pair_locus, d.pair_mask, d.count)
-    assert hp.relerr(theta, eo.prepare(oapm, eff, 0.0)) < 1e-12
+    where = layouts.locus_kinds(pat.packed)
+    xr.assert_elementwise(theta, x.prepare(eff), x.rtol_prepare(), "theta0", where)
     for model in (4, 3, 4):
-        want = eo.sum_read(oapm, eo.e_step(oapm, theta, model, gene_of))
+        counts, _ = x.update(theta, model, eff)
         out = pat.run(model, tol=0.0, max_iters=1)
-        assert out["iters"] == 1 and hp.relerr(out["counts"], want) < 1e-12
+        assert out["iters"] == 1
+        xr.assert_elementwise(out["counts"], counts, x.rtol_update(model), f"model {model} counts", where)
         theta = out["theta"]
+
+
+@pytest.mark.parametrize("H", range(1, 9))
+def test_emulated_elementwise_on_constructed_layouts(H):
+    """One update of every model from a haplotype-asymmetric theta scattered over e^+-40 (some in-support slots exactly 0),
+    on a layout that reaches every column-pass segment, row-pass width and lane mask of H haplotypes: expected counts and
+    theta element by element against the extended-precision reference, within the error bound of tests/xref.py.  A theta'
+    flushed to zero, a lost or doubled entry, a swapped haplotype: any of them fails here whatever its magnitude."""
+    import ctypes as C
+
+    xr.require_longdouble()
+    d = layouts.make_layout(H)
+    gene_of = eo.gene_index(d.T, d.groups())
+    pat = simt_em.HostPattern(synth.to_apm(d), gene_of=gene_of, item_len=16)
+    layouts.assert_layout_covers(pat.packed)
+    where = layouts.locus_kinds(pat.packed)
+    x = xr.XRef(d, gene_of)
+    eff = eo.effective_length_table(d.lengths)
+    xr.assert_elementwise(pat.prepare(eff), x.prepare(eff), x.rtol_prepare(), "theta0", where)
+    theta = xr.random_theta(x, seed=H)
+    tb = np.zeros((d.T, 8))  # referenced until the end: the library reads it through a raw pointer
+    tb[:, :H] = theta.T
+    for model in (4, 3, 2, 1):
+        pat.check(pat.lib.gbrs_em_set_theta(C.byref(pat.desc), tb.ctypes.data, None))
+        out = pat.run(model, tol=0.0, max_iters=1)
+        counts, theta1 = x.update(theta, model, eff)
+        rtol = x.rtol_update(model)
+        xr.assert_elementwise(out["counts"], counts, rtol, f"H={H} model {model} counts", where)
+        xr.assert_elementwise(out["theta"], theta1, rtol, f"H={H} model {model} theta", where)
+        assert not out["counts"][:, d.zero_locus].any()
 
 
 def test_emulated_standalone_estep_does_not_move_the_state():
