@@ -16,7 +16,10 @@ seven column-pass segments.
 
 `assert_layout_covers(packed)` reads the pack info, the width buckets and the item_desc trailer and fails if a kind of work
 is missing.  Every test on a constructed layout calls it: if the packer or the constructor drifts, the test fails instead of
-quietly covering less."""
+quietly covering less.
+
+`make_empty_shards(kind, R)` builds inputs for which the class split of the packer leaves some of R row shards without a
+class; `assert_empty_shards` checks that it did."""
 from __future__ import annotations
 
 import numpy as np
@@ -132,6 +135,48 @@ def make_layout(H: int, item_len: int = 16, seed: int = 0) -> synth.SynthData:
     assert set(WIDTHS) <= set(widths.tolist())
     assert np.all(count[np.unique(pair_class[pair_locus == z_locus])] == 0)
     return d
+
+
+def make_heavy_first_class(T: int, seed: int = 0) -> synth.SynthData:
+    """Class 0 hits every locus with a full mask of 8 haplotypes; the other T // 2 classes are single pairs of one
+    haplotype.  Class 0 holds 16/17 of the nnz, more than (R - 1) / R for any R <= 8, so the packer's class split (class c
+    to rank floor(cum_before(c) R / nnz)) sends class 0 to rank 0, everything else to rank R - 1 and nothing in between."""
+    rng = np.random.default_rng(seed)
+    n_small = T // 2
+    pc = [0] * T + list(range(1, n_small + 1))
+    pl = list(range(T)) + [int(t) for t in rng.integers(0, T, n_small)]
+    pm = [0xFF] * T + [1 << int(h) for h in rng.integers(0, 8, n_small)]
+    d = synth.SynthData(T=T, H=8, N=n_small + 1, pair_class=np.array(pc, np.int64), pair_locus=np.array(pl, np.int64),
+                        pair_mask=np.array(pm, np.uint8), count=rng.integers(1, 20, n_small + 1).astype(np.float64),
+                        gene_of=np.repeat(np.arange(T), 3)[:T].astype(np.int64),
+                        lengths=rng.integers(300, 6000, size=(T, 8)).astype(np.float64), hname=synth.HAPLOTYPES[:8])
+    d.lname = [f"T{t:04d}" for t in range(T)]
+    d.gname = [f"G{g:04d}" for g in range(int(d.gene_of.max()) + 1)]
+    return d
+
+
+def make_empty_shards(kind: str, R: int) -> synth.SynthData:
+    """An input that leaves some of R row shards without any class: "few classes" (fewer classes than ranks) or "heavy
+    first class" (make_heavy_first_class)."""
+    if kind == "few classes":
+        return synth.generate(T=6, N=max(1, R - 3), H=8, sample_index=4)
+    if kind == "heavy first class":
+        return make_heavy_first_class(T=20, seed=R)
+    raise ValueError(kind)
+
+
+def assert_empty_shards(kind: str, d, classes, nnz) -> None:
+    """`classes` / `nnz`: per shard, from the pack info.  The shards hold all of the nnz, and the ranks the input was built
+    to leave empty really have no class."""
+    R = len(classes)
+    nnz = [int(n) for n in nnz]
+    assert sum(nnz) == d.nnz, (nnz, d.nnz)
+    empty = [r for r, c in enumerate(classes) if c == 0]
+    assert all(nnz[r] == 0 for r in empty)
+    if kind == "few classes":
+        assert d.N < R and len(empty) >= R - d.N, classes
+    else:
+        assert empty == list(range(1, R - 1)) and classes[0] == 1, classes
 
 
 def layout_summary(info, item_desc) -> dict:
