@@ -15,7 +15,7 @@ LIB_PATH = os.environ.get("GBRS_LIB_PATH") or os.path.join(HERE, "_C", "libgbrs_
 GBRS_HPAD = 8
 GBRS_KMAX = 8
 GBRS_PART_SLOTS = 4096
-ABI_VERSION = 6
+ABI_VERSION = 7
 CTRL_ITERS, CTRL_DONE, CTRL_ERROR, CTRL_PARITY, CTRL_MAX_ITERS, CTRL_PREPARED = range(6)
 SCAL_ERR, SCAL_SUM_PREV, SCAL_TARGET, SCAL_SUM_CUR = range(4)
 
@@ -47,8 +47,8 @@ class PackInfo(C.Structure):
 
 
 class DevicePack(C.Structure):
-    _fields_ = [(n, C.c_void_p) for n in ("rowptr", "pairs", "count", "runptr", "ent_cls", "ent_pair", "ent_run", "item_desc",
-                                          "locus_desc", "gene_of", "gene_ptr", "gene_loci")]
+    _fields_ = [(n, C.c_void_p) for n in ("rowptr", "pairs", "count", "runptr", "class_id", "ent_cls", "ent_pair", "ent_run",
+                                          "item_desc", "locus_desc", "gene_of", "gene_ptr", "gene_loci")]
 
 
 ALLOC_FN = C.CFUNCTYPE(C.c_void_p, C.c_int64, C.c_char_p, C.c_void_p)
@@ -137,6 +137,11 @@ SYMBOLS = {
     "gbrs_em_run_cb": (C.c_int, [C.POINTER(EmDev), C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p,
                                  C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p]),
     "gbrs_em_read_ctrl": (C.c_int, [C.POINTER(EmDev), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gbrs_em_posterior_scratch_bytes": (C.c_int, [C.POINTER(EmDev), C.c_int, C.c_int64, C.POINTER(C.c_int64)]),
+    "gbrs_em_posterior": (C.c_int, [C.POINTER(EmDev), C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_void_p),
+                                    C.POINTER(C.c_void_p), C.c_int32, C.POINTER(C.c_void_p), C.c_void_p, C.c_int64,
+                                    C.c_void_p]),
+    "gbrs_em_copy_theta": (C.c_int, [C.POINTER(EmDev), C.c_int, C.c_void_p, C.c_void_p]),
     "gbrs_write_table": (C.c_int, [C.c_char_p, C.c_char_p, C.POINTER(C.c_char_p), C.c_int64, C.c_void_p, C.c_int32,
                                    C.POINTER(C.c_char_p), C.c_void_p, C.c_int32]),
     "gbrs_parse_lengths": (C.c_int, [C.c_char_p, C.POINTER(C.c_char_p), C.c_int64, C.POINTER(C.c_char_p), C.c_int32,

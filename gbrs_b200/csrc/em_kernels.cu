@@ -2271,6 +2271,203 @@ inline gbrs_em_dev locus_view(const gbrs_em_dev* d, bool tiles) {
   return v;
 }
 
+// Row pass (E-step weights) of `model` on the two-pass layout, for d->n_classes > 0: the launches of an EM update, shared by
+// the update (launch_local_impl) and the posterior (gbrs_em_posterior).  Model 4 reads the subset tables, models 1-3 the
+// gene totals too (k_gene_totals before this).
+int launch_row_pass(const gbrs_em_dev* d, int model, cudaStream_t s) {
+  switch (model) {
+    case 4: if (int rc4 = launch_row_m4<false>(d, s)) return rc4; break;
+    case 3:
+    case 2: {
+      const int64_t n_fixed = d->bucket_class0[GBRS_KMAX], n_long = d->n_classes - n_fixed;
+      if (n_fixed > 0) {  // wide classes first, then the narrow ones at their own (smaller) register budget
+        int rcf = model == 3 ? launch_m23_fixed<3, 4, GBRS_KMAX>(d, s) : launch_m23_fixed<2, 4, GBRS_KMAX>(d, s);
+        if (!rcf) rcf = model == 3 ? launch_m23_fixed<3, 1, 3>(d, s) : launch_m23_fixed<2, 1, 3>(d, s);
+        if (rcf) return rcf;
+      }
+      if (n_long > 0) {
+        if (model == 3) k_weights_m3<<<grid_for(n_long), kThreads, 0, s>>>(*d, n_fixed);
+        else k_weights_m2<<<grid_for(n_long), kThreads, 0, s>>>(*d, n_fixed);
+      }
+      break;
+    }
+    default: {
+      // GBRS_M1_FIXED: eight lanes per class for the classes of up to GBRS_KMAX pairs (parity-tested, not yet timed)
+      static const bool m1_fixed = std::getenv("GBRS_M1_FIXED") != nullptr;
+      static const bool m1_generic = std::getenv("GBRS_M1_GENERIC") != nullptr;  // A/B knob: the round-1 row pass for all
+      if (!m1_fixed && !m1_generic) {
+        // default: narrow classes thread-per-class without row pointers, the rest through the generic CSR walk
+        const int64_t n_narrow = d->bucket_class0[kM1Narrow], n_rest = d->n_classes - n_narrow;
+        if (n_rest > 0) k_weights_m1<<<grid_for(n_rest), kThreads, 0, s>>>(*d, n_narrow);
+        int rcn = launch_m1_narrow<3>(d, s);
+        if (!rcn) rcn = launch_m1_narrow<2>(d, s);
+        if (!rcn) rcn = launch_m1_narrow<1>(d, s);
+        if (rcn) return rcn;
+        break;
+      }
+      const int64_t n_fixed = m1_fixed ? d->bucket_class0[GBRS_KMAX] : 0, n_long = d->n_classes - n_fixed;
+      if (n_fixed > 0) {  // widest first
+        int r8 = launch_m1_fixed<8>(d, s);
+        if (!r8) r8 = launch_m1_fixed<7>(d, s);
+        if (!r8) r8 = launch_m1_fixed<6>(d, s);
+        if (!r8) r8 = launch_m1_fixed<5>(d, s);
+        if (!r8) r8 = launch_m1_fixed<4>(d, s);
+        if (!r8) r8 = launch_m1_fixed<3>(d, s);
+        if (!r8) r8 = launch_m1_fixed<2>(d, s);
+        if (!r8) r8 = launch_m1_fixed<1>(d, s);
+        if (r8) return r8;
+      }
+      if (n_long > 0) k_weights_m1<<<grid_for(n_long), kThreads, 0, s>>>(*d, n_fixed);
+      break;
+    }
+  }
+  GBRS_LAUNCH_CHECK("k_weights");
+  return GBRS_OK;
+}
+
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Posterior P[n,t,h] of one E-step on an output pattern (gbrs_em_posterior).  The row pass of the model runs unmodified on
+// a copy of the descriptor whose theta is theta_src, whose counts are ones and whose work tables are scratch; then, since
+// count_n P[n,t,h] = theta[t][h] W[idx(n,t,h)] (k_locus_acc sums exactly these products), every entry of the output CSC
+// is theta_src[t][h] times one weight.  Error codes in ctrl[GBRS_CTRL_ERROR] of the scratch copy: 1 = zero normaliser or
+// non-finite value, 2 = the output pattern is not the packed one.
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr uint32_t kNoClass = 0xFFFFFFFFu;
+
+__global__ void __launch_bounds__(kThreads) k_post_init(int64_t N, uint32_t* class_pos, int64_t n_classes, double* ones) {
+  const int64_t stride = (int64_t) gridDim.x * blockDim.x;
+  const int64_t n = N > n_classes ? N : n_classes;
+  for (int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    if (i < N) class_pos[i] = kNoClass;
+    if (i < n_classes) ones[i] = 1.0;
+  }
+}
+
+// class_pos = inverse of the packer's class order (input class id -> packed class)
+__global__ void __launch_bounds__(kThreads) k_post_class_pos(int64_t n_classes, const uint32_t* __restrict__ class_id, int64_t N,
+                                                             uint32_t* __restrict__ class_pos, int32_t* ctrl) {
+  const int64_t stride = (int64_t) gridDim.x * blockDim.x;
+  for (int64_t p = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; p < n_classes; p += stride) {
+    const uint32_t c = __ldg(class_id + p);
+    if ((int64_t) c < N) class_pos[c] = (uint32_t) p;
+    else atomicMax(ctrl + GBRS_CTRL_ERROR, 2);
+  }
+}
+
+// Models 1-3 guard their divisions, so a class whose entries all have theta 0 gets weights 0 instead of 0 / 0.  Every
+// normaliser of such a class is 0 exactly when the sum of theta over its entries is (each is bounded below by one of its
+// non-zero terms): that sum, from the subset tables of theta_src.
+__global__ void __launch_bounds__(kThreads) k_post_dead_classes(const gbrs_em_dev d) {
+  const int64_t stride = (int64_t) gridDim.x * blockDim.x;
+  for (int64_t n = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; n < d.n_classes; n += stride) {
+    const uint32_t b = __ldg(d.rowptr + n), e = __ldg(d.rowptr + n + 1);
+    double s = 0.0;
+    for (uint32_t p = b; p < e; ++p) s += pair_sum(d.subsets, __ldg(d.pairs + p));
+    if (!(s > 0.0)) atomicMax(d.ctrl + GBRS_CTRL_ERROR, 1);
+  }
+}
+
+// One warp per locus column of haplotype h, lanes over its entries (consecutive: coalesced index loads and value stores).
+// idx of the entry's weight: the packed class (model 4); otherwise its pair in the class' row, found by a walk over the
+// row (pairs sorted by (gene, locus)) that counts the gene runs on the way (model 3: the run, model 1: run * 8 + h).
+template <typename I, int MODEL>
+__global__ void __launch_bounds__(kThreads) k_post_gather(const gbrs_em_dev d, int h, int64_t N, const uint32_t* __restrict__ class_pos,
+                                                          const int64_t* __restrict__ indptr, const I* __restrict__ indices,
+                                                          double* __restrict__ values) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = ((int64_t) gridDim.x * blockDim.x) >> 5;
+  const double* __restrict__ th = d.theta;  // theta_src (parity 0 of the scratch control block)
+  int err = 0;
+  for (int64_t t = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5; t < d.T; t += nwarps) {
+    const int64_t b = __ldg(indptr + t), e = __ldg(indptr + t + 1);
+    if (b == e) continue;
+    const double x = __ldg(th + (size_t) t * GBRS_HPAD + h);
+    for (int64_t i = b + lane; i < e; i += 32) {
+      const int64_t n = (int64_t) __ldg(indices + i);
+      const uint32_t p = (n >= 0 && n < N) ? __ldg(class_pos + n) : kNoClass;
+      double v = 0.0;
+      if (n < 0 || n >= N) {
+        err = 2;
+      } else if (p != kNoClass) {
+        size_t idx = p;
+        if (MODEL != 4) {
+          const uint32_t rb = __ldg(d.rowptr + p), re = __ldg(d.rowptr + p + 1);
+          uint32_t q = rb, run = MODEL == 2 ? 0u : __ldg(d.runptr + p), w = 0u;
+          int32_t g_prev = 0;
+          for (; q < re; ++q) {
+            w = __ldg(d.pairs + q);
+            const uint32_t tl = w & kLocusMask;
+            if (MODEL != 2) {
+              const int32_t g = __ldg(d.gene_of + tl);
+              if (q > rb && g != g_prev) ++run;
+              g_prev = g;
+            }
+            if ((int64_t) tl == t) break;
+          }
+          idx = MODEL == 2 ? (size_t) q : (MODEL == 3 ? (size_t) run : (size_t) run * GBRS_HPAD + h);
+          if (q == re || !((w >> (24 + h)) & 1u)) {
+            err = 2;
+            idx = 0;
+          }
+        }
+        v = x * d.weights[idx];
+        if (!isfinite(v) && err == 0) err = 1;
+      }
+      values[i] = v;
+    }
+  }
+  if (err) atomicMax(d.ctrl + GBRS_CTRL_ERROR, err);
+}
+
+template <typename I>
+int launch_post_gather(const gbrs_em_dev* v, int model, int h, int64_t N, const uint32_t* class_pos, const int64_t* indptr,
+                       const void* indices, double* values, cudaStream_t s) {
+  const I* ix = static_cast<const I*>(indices);
+  const int64_t threads = (int64_t) v->T * 32;
+  switch (model) {
+    case 4: k_post_gather<I, 4><<<resident_grid(k_post_gather<I, 4>, threads), kThreads, 0, s>>>(*v, h, N, class_pos, indptr, ix, values); break;
+    case 3: k_post_gather<I, 3><<<resident_grid(k_post_gather<I, 3>, threads), kThreads, 0, s>>>(*v, h, N, class_pos, indptr, ix, values); break;
+    case 2: k_post_gather<I, 2><<<resident_grid(k_post_gather<I, 2>, threads), kThreads, 0, s>>>(*v, h, N, class_pos, indptr, ix, values); break;
+    default: k_post_gather<I, 1><<<resident_grid(k_post_gather<I, 1>, threads), kThreads, 0, s>>>(*v, h, N, class_pos, indptr, ix, values); break;
+  }
+  GBRS_LAUNCH_CHECK("k_post_gather");
+  return GBRS_OK;
+}
+
+// scratch of gbrs_em_posterior: byte offsets (each 256-byte aligned)
+struct PostScratch {
+  int64_t ctrl, part, iso, subsets, gene_hap, gamma, count, weights, class_pos, total;
+};
+inline PostScratch post_scratch(const gbrs_em_dev* d, int model, int64_t N) {
+  auto up = [](int64_t b) { return (b + 255) & ~int64_t(255); };
+  const int64_t runs = d->n_runs, T = d->T;
+  int64_t wlen = d->n_classes > d->n_pairs ? d->n_classes : d->n_pairs;
+  if (runs > wlen) wlen = runs;
+  if (model == 1 && 8 * runs > wlen) wlen = 8 * runs;
+  wlen += 8;
+  PostScratch L;
+  int64_t o = 0;
+  L.ctrl = o;      o += up(16 * sizeof(int32_t));
+  L.part = o;      o += up(GBRS_PART_SLOTS * sizeof(double));
+  L.iso = o;       o += up(T * sizeof(double));
+  L.subsets = o;   o += up(T * 32 * sizeof(double));
+  L.gene_hap = o;  o += up((int64_t) (d->n_gene_ids > 1 ? d->n_gene_ids : 1) * GBRS_HPAD * sizeof(double));
+  L.gamma = o;     o += up(T * sizeof(double));
+  L.count = o;     o += up((d->n_classes > 1 ? d->n_classes : 1) * sizeof(double));
+  L.weights = o;   o += up(wlen * sizeof(double));
+  L.class_pos = o; o += up((N > 1 ? N : 1) * sizeof(uint32_t));
+  L.total = o;
+  return L;
+}
+
+__global__ void __launch_bounds__(kThreads) k_copy_theta(const gbrs_em_dev d, int previous, double* dst) {
+  const double* __restrict__ src = d.theta + (size_t) (d.ctrl[GBRS_CTRL_PARITY] ^ previous) * d.T * GBRS_HPAD;
+  const int64_t total = (int64_t) d.T * GBRS_HPAD;
+  const int64_t stride = (int64_t) gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) dst[i] = src[i];
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -2470,53 +2667,7 @@ static int launch_local_impl(const gbrs_em_dev* d, int model, void* stream, gbrs
   if (tiles) {
     if (int rct = launch_tiles<false>(d, s)) return rct;
   } else if (d->n_classes > 0) {
-    switch (model) {
-      case 4: if (int rc4 = launch_row_m4<false>(d, s)) return rc4; break;
-      case 3:
-      case 2: {
-        const int64_t n_fixed = d->bucket_class0[GBRS_KMAX], n_long = d->n_classes - n_fixed;
-        if (n_fixed > 0) {  // wide classes first, then the narrow ones at their own (smaller) register budget
-          int rcf = model == 3 ? launch_m23_fixed<3, 4, GBRS_KMAX>(d, s) : launch_m23_fixed<2, 4, GBRS_KMAX>(d, s);
-          if (!rcf) rcf = model == 3 ? launch_m23_fixed<3, 1, 3>(d, s) : launch_m23_fixed<2, 1, 3>(d, s);
-          if (rcf) return rcf;
-        }
-        if (n_long > 0) {
-          if (model == 3) k_weights_m3<<<grid_for(n_long), kThreads, 0, s>>>(*d, n_fixed);
-          else k_weights_m2<<<grid_for(n_long), kThreads, 0, s>>>(*d, n_fixed);
-        }
-        break;
-      }
-      default: {
-        // GBRS_M1_FIXED: eight lanes per class for the classes of up to GBRS_KMAX pairs (parity-tested, not yet timed)
-        static const bool m1_fixed = std::getenv("GBRS_M1_FIXED") != nullptr;
-        static const bool m1_generic = std::getenv("GBRS_M1_GENERIC") != nullptr;  // A/B knob: the round-1 row pass for all
-        if (!m1_fixed && !m1_generic) {
-          // default: narrow classes thread-per-class without row pointers, the rest through the generic CSR walk
-          const int64_t n_narrow = d->bucket_class0[kM1Narrow], n_rest = d->n_classes - n_narrow;
-          if (n_rest > 0) k_weights_m1<<<grid_for(n_rest), kThreads, 0, s>>>(*d, n_narrow);
-          int rcn = launch_m1_narrow<3>(d, s);
-          if (!rcn) rcn = launch_m1_narrow<2>(d, s);
-          if (!rcn) rcn = launch_m1_narrow<1>(d, s);
-          if (rcn) return rcn;
-          break;
-        }
-        const int64_t n_fixed = m1_fixed ? d->bucket_class0[GBRS_KMAX] : 0, n_long = d->n_classes - n_fixed;
-        if (n_fixed > 0) {  // widest first
-          int r8 = launch_m1_fixed<8>(d, s);
-          if (!r8) r8 = launch_m1_fixed<7>(d, s);
-          if (!r8) r8 = launch_m1_fixed<6>(d, s);
-          if (!r8) r8 = launch_m1_fixed<5>(d, s);
-          if (!r8) r8 = launch_m1_fixed<4>(d, s);
-          if (!r8) r8 = launch_m1_fixed<3>(d, s);
-          if (!r8) r8 = launch_m1_fixed<2>(d, s);
-          if (!r8) r8 = launch_m1_fixed<1>(d, s);
-          if (r8) return r8;
-        }
-        if (n_long > 0) k_weights_m1<<<grid_for(n_long), kThreads, 0, s>>>(*d, n_fixed);
-        break;
-      }
-    }
-    GBRS_LAUNCH_CHECK("k_weights");
+    if (int rcr = launch_row_pass(d, model, s)) return rcr;
   }
   }
   if (ev) GBRS_CUDA(cudaEventRecord(ev[1], s));
@@ -2717,5 +2868,107 @@ extern "C" int gbrs_em_alignment_counts(const gbrs_em_dev* d, int gene_level, in
   k_alignment_counts<<<grid_for(d->n_classes), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       *d, gene_level, n_real_genes, aln_dev, uniq_dev, locus_uniq_dev);
   GBRS_LAUNCH_CHECK("k_alignment_counts");
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_em_posterior_scratch_bytes(const gbrs_em_dev* d, int model, int64_t N, int64_t* bytes) {
+  if (!d || !bytes || model < 1 || model > 4 || N < 0) { gbrs_set_error("gbrs_em_posterior_scratch_bytes: bad argument"); return GBRS_E_ARG; }
+  *bytes = post_scratch(d, model, N).total;
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_em_posterior(const gbrs_em_dev* d, int model, const double* theta_src, const uint32_t* class_id, int64_t N,
+                                 const int64_t* const* indptr, const void* const* indices, int32_t index_bytes,
+                                 double* const* values, void* scratch, int64_t scratch_bytes, void* stream) {
+  const char* who = "gbrs_em_posterior";
+  if (!d) { gbrs_set_error("gbrs_em_posterior: null descriptor"); return GBRS_E_ARG; }
+  if (model < 1 || model > 4) { gbrs_set_error("The read normalization model should be 1, 2, 3, or 4."); return GBRS_E_ARG; }
+  if (d->T <= 0 || d->H < 1 || d->H > GBRS_HPAD || N < 0 || N >= (int64_t(1) << 32) || (index_bytes != 4 && index_bytes != 8) ||
+      !theta_src || !indptr || !indices || !values || !scratch) {
+    gbrs_set_error("gbrs_em_posterior: bad argument"); return GBRS_E_ARG;
+  }
+  for (int h = 0; h < d->H; ++h)
+    if (!indptr[h] || !indices[h] || !values[h]) { gbrs_set_error("gbrs_em_posterior: null output pattern array"); return GBRS_E_ARG; }
+  if (d->n_classes > 0 && (!d->pairs || !class_id)) { gbrs_set_error("gbrs_em_posterior: pairs / class_id missing"); return GBRS_E_ARG; }
+  if (model != 4 && (!d->gene_of || !d->gene_ptr || !d->gene_loci || !d->rowptr || !d->runptr)) {
+    gbrs_set_error("gbrs_em_posterior: models 1-3 need rowptr / runptr and the gene tables"); return GBRS_E_ARG;
+  }
+  const PostScratch L = post_scratch(d, model, N);
+  if (scratch_bytes < L.total) { gbrs_set_error("gbrs_em_posterior: scratch too small"); return GBRS_E_ARG; }
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) { gbrs_set_error(std::string(who) + ": no CUDA device (there is no CPU fallback)"); return GBRS_E_CUDA; }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  char* base = static_cast<char*>(scratch);
+  uint32_t* class_pos = reinterpret_cast<uint32_t*>(base + L.class_pos);
+  // the row pass' view: theta_src at parity 0 of a zeroed control block, unit counts, own tables -- one rank, no tiles
+  gbrs_em_dev v = *d;
+  v.theta = const_cast<double*>(theta_src);
+  v.ctrl = reinterpret_cast<int32_t*>(base + L.ctrl);
+  v.part = reinterpret_cast<double*>(base + L.part);
+  v.iso = reinterpret_cast<double*>(base + L.iso);
+  v.subsets = reinterpret_cast<double*>(base + L.subsets);
+  v.gene_hap = reinterpret_cast<double*>(base + L.gene_hap);
+  v.gamma = reinterpret_cast<double*>(base + L.gamma);
+  double* ones = reinterpret_cast<double*>(base + L.count);
+  v.count = ones;
+  v.weights = reinterpret_cast<double*>(base + L.weights);
+  v.acc = v.wit = v.err_log = v.scal = nullptr;  // the EM's buffers: nothing here writes them
+  v.xchg_enabled = 0;
+  v.n_ranks = 1;
+  v.xchg_mc = nullptr;
+  v.tile_blob = nullptr;
+  v.tile_desc = v.tile_locus_desc = nullptr;
+  v.tile_partial = nullptr;
+  GBRS_CUDA(cudaMemsetAsync(v.ctrl, 0, 16 * sizeof(int32_t), s));
+  const int64_t n_init = N > d->n_classes ? N : d->n_classes;
+  if (n_init > 0) {
+    k_post_init<<<grid_for(n_init), kThreads, 0, s>>>(N, class_pos, d->n_classes, ones);
+    GBRS_LAUNCH_CHECK("k_post_init");
+  }
+  if (d->n_classes > 0) {
+    k_post_class_pos<<<grid_for(d->n_classes), kThreads, 0, s>>>(d->n_classes, class_id, N, class_pos, v.ctrl);
+    GBRS_LAUNCH_CHECK("k_post_class_pos");
+  }
+  k_subset_tables<<<resident_grid(k_subset_tables, (int64_t) d->T * 32), kThreads, 0, s>>>(v);
+  GBRS_LAUNCH_CHECK("k_subset_tables");
+  if (model == 2) {  // isoform totals of theta_src (into iso[0]), summed as the EM sums them
+    k_locus_update<false><<<locus_grid(&v), kThreads, 0, s>>>(v);
+    GBRS_LAUNCH_CHECK("k_locus_update<refresh>");
+  }
+  if (model != 4) {
+    k_gene_totals<<<grid_for((int64_t) d->n_gene_ids * 8), kThreads, 0, s>>>(v);
+    GBRS_LAUNCH_CHECK("k_gene_totals");
+  }
+  if (d->n_classes > 0) {
+    if (int rc = launch_row_pass(&v, model, s)) return rc;
+    if (model != 4) {
+      k_post_dead_classes<<<grid_for(d->n_classes), kThreads, 0, s>>>(v);
+      GBRS_LAUNCH_CHECK("k_post_dead_classes");
+    }
+  }
+  for (int h = 0; h < d->H; ++h) {
+    const int rc = index_bytes == 4 ? launch_post_gather<uint32_t>(&v, model, h, N, class_pos, indptr[h], indices[h], values[h], s)
+                                    : launch_post_gather<unsigned long long>(&v, model, h, N, class_pos, indptr[h], indices[h], values[h], s);
+    if (rc) return rc;
+  }
+  int32_t ctrl[16];
+  GBRS_CUDA(cudaMemcpyAsync(ctrl, v.ctrl, sizeof(ctrl), cudaMemcpyDeviceToHost, s));
+  GBRS_CUDA(cudaStreamSynchronize(s));
+  if (ctrl[GBRS_CTRL_ERROR] == 2) {
+    gbrs_set_error("gbrs_em_posterior: the output pattern holds an entry the packed incidence does not");
+    return GBRS_E_ARG;
+  }
+  if (ctrl[GBRS_CTRL_ERROR]) {
+    gbrs_set_error("non-finite posterior probability (a class with a zero normaliser)");
+    return GBRS_E_NUMERIC;
+  }
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_em_copy_theta(const gbrs_em_dev* d, int previous, double* dst, void* stream) {
+  if (int rc = check_dev(d, "gbrs_em_copy_theta")) return rc;
+  if (!dst || (previous != 0 && previous != 1)) { gbrs_set_error("gbrs_em_copy_theta: bad argument"); return GBRS_E_ARG; }
+  k_copy_theta<<<grid_for((int64_t) d->T * GBRS_HPAD), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(*d, previous, dst);
+  GBRS_LAUNCH_CHECK("k_copy_theta");
   return GBRS_OK;
 }

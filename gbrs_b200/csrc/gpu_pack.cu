@@ -739,6 +739,7 @@ extern "C" int gbrs_pack_device(const gbrs_pack_input* in, gbrs_alloc_fn alloc, 
   uint32_t* rowptr = A.get<uint32_t>(n_classes + 1, "rowptr");
   uint32_t* runptr = A.get<uint32_t>(n_classes + 1, "runptr");
   double* count = A.get<double>(n_classes, "count");
+  uint32_t* class_id = A.get<uint32_t>(n_classes, "class_id");
   uint32_t* npair_new = A.get<uint32_t>(n_classes + 1, "tmp:npair_new");
   uint32_t* nruns = A.get<uint32_t>(n_classes + 1, "tmp:nruns");
   if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
@@ -746,6 +747,8 @@ extern "C" int gbrs_pack_device(const gbrs_pack_input* in, gbrs_alloc_fn alloc, 
   GP_CUDA(cudaMemsetAsync(runptr, 0, sizeof(uint32_t), s));
   uint32_t n_pairs32 = 0, n_runs32 = 0;
   if (n_classes > 0) {
+    // the first n_classes entries of the order are this shard's non-empty classes: their input ids are the class ids
+    GP_CUDA(cudaMemcpyAsync(class_id, order, sizeof(uint32_t) * (size_t) n_classes, cudaMemcpyDeviceToDevice, s));
     k_gp_gather_u32<<<gp_grid(n_classes), kGpThreads, 0, s>>>(n_classes, order, npair, npair_new);
     if (int rc = inclusive_scan_into(A, npair_new, rowptr + 1, n_classes, s)) return rc;
     if (int rc = read_back(rowptr + n_classes, &n_pairs32, 1, s)) return rc;
@@ -842,6 +845,7 @@ extern "C" int gbrs_pack_device(const gbrs_pack_input* in, gbrs_alloc_fn alloc, 
   out->pairs = pairs;
   out->count = count;
   out->runptr = runptr;
+  out->class_id = class_id;
   out->item_desc = item_desc;
   out->locus_desc = locus_desc;
   out->gene_of = d_gene_of;

@@ -247,10 +247,12 @@ extern "C" int gbrs_pack_create(const gbrs_pack_input* in, gbrs_pack_t* out) {
     P->H = H;
     par_fill(P->rowptr, (size_t) n_classes + 1, 0u);
     par_fill(P->count, (size_t) n_classes, 1.0);
+    P->class_id.resize((size_t) n_classes);  // every slot is written below (new_id is a bijection onto [0, n_classes))
 #pragma omp parallel for schedule(static)
     for (int64_t c = lo; c < hi; ++c)
       if (npair[c]) {
         P->rowptr[new_id[c] + 1] = npair[c];
+        P->class_id[new_id[c]] = (uint32_t) c;
         if (in->count) P->count[new_id[c]] = in->count[c];
       }
     for (int64_t n = 0; n < n_classes; ++n) P->rowptr[n + 1] += P->rowptr[n];
@@ -568,6 +570,7 @@ extern "C" int gbrs_pack_get_array(gbrs_pack_t p, const char* name, const void**
   GBRS_ARR("pairs", p->pairs)
   GBRS_ARR("count", p->count)
   GBRS_ARR("runptr", p->runptr)
+  GBRS_ARR("class_id", p->class_id)
   GBRS_ARR("ent_cls", p->ent_cls)
   GBRS_ARR("ent_pair", p->ent_pair)
   GBRS_ARR("ent_run", p->ent_run)

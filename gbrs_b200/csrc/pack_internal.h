@@ -45,6 +45,7 @@ struct gbrs_pack {
   gbrs_pack_info info{};
   int32_t T = 0, H = 0;
   bigvec<uint32_t> rowptr, pairs, runptr;
+  bigvec<uint32_t> class_id;  // [n_classes] input class id of every packed class
   std::vector<uint32_t> item_off, item_order, item_desc, locus_item_ptr, locus_order, locus_desc, gene_ptr, gene_loci;
   std::vector<int32_t> gene_of;
   bigvec<double> count;

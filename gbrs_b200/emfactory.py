@@ -11,10 +11,11 @@ exchange step of a row-sharded run (sum of the T x H numerator).  There is no CP
 library or without a CUDA device every compute call raises.
 
 Differences from the reference that a caller can observe (DESIGN.md section 6):
-  * the posterior P[n,t,h] is never materialised; after `run`, `self.probability` still holds the incidence pattern.
+  * the EM never materialises the posterior P[n,t,h]; after `run`, `self.probability` still holds the incidence pattern.
     Expected read counts come from the device-side numerator (identical to `probability.sum(READ)` of the last
-    posterior).
-  * classes are re-ordered internally; nothing class-indexed is returned, so this is invisible.
+    posterior).  `posterior_probability()` computes, on request, the matrix the reference's `probability` holds after
+    the last call: a new `AlignmentPropertyMatrix` with P on the EM's pattern (DESIGN.md section 7.1).
+  * classes are re-ordered internally; class-indexed results are returned in the input's class order.
 """
 from __future__ import annotations
 
@@ -32,7 +33,7 @@ logger = utils.get_logger("gbrs")
 ERR_LOG_CAP = 1 << 16
 
 _PACK_ARRAYS = {  # name -> numpy dtype (None = entry word, depends on entry_bytes)
-    "rowptr": np.uint32, "pairs": np.uint32, "count": np.float64, "runptr": np.uint32,
+    "rowptr": np.uint32, "pairs": np.uint32, "count": np.float64, "runptr": np.uint32, "class_id": np.uint32,
     "ent_cls": None, "ent_pair": None, "ent_run": None, "item_off": np.uint32, "item_order": np.uint32, "item_desc": np.uint32, "locus_order": np.uint32, "locus_desc": np.uint32,
     "locus_item_ptr": np.uint32,
     "gene_ptr": np.uint32, "gene_loci": np.uint32, "gene_of": np.int32,
@@ -44,6 +45,8 @@ _PACK_ARRAYS = {  # name -> numpy dtype (None = entry word, depends on entry_byt
 # read by a kernel.
 _LAZY_ARRAYS = ("rowptr", "runptr", "ent_pair", "ent_run")
 _HOST_ONLY_ARRAYS = ("item_off", "item_order", "locus_order", "locus_item_ptr")
+# Read by the posterior only (gbrs_em_posterior): uploaded by its first call, never by an EM run.
+_POSTERIOR_ARRAYS = ("class_id",)
 
 
 _STAGING: dict = {}  # (device, T) -> pinned [T][8] staging buffer shared by the patterns of a process (used synchronously)
@@ -111,6 +114,26 @@ def pack_input(apm: APM, gene_of=None, hapmask=None, shard_rank=0, shard_count=1
     inp.shard_rank, inp.shard_count, inp.item_len = shard_rank, shard_count, item_len
     keep += [count, hapmask, gene_of]
     return inp, keep
+
+
+def posterior_pattern(apm: APM, hapmask=None) -> list:
+    """Per haplotype (indptr int64, indices, stored values) of the pattern the EM runs on: the input CSC in canonical form
+    (sorted indices, duplicates summed), with the (t, h) columns a genotype restriction `hapmask` removes emptied."""
+    out = []
+    for h, m in enumerate(apm.data):
+        m = m if m.format == "csc" else m.tocsc()
+        if not m.has_canonical_format:
+            m = m.copy()
+            m.sum_duplicates()
+        indptr, indices, data = np.asarray(m.indptr, dtype=np.int64), m.indices, m.data
+        if hapmask is not None:
+            keep = ((np.asarray(hapmask) >> h) & 1).astype(bool)
+            lens = np.diff(indptr)
+            sel = np.repeat(keep, lens)
+            indices, data = indices[sel], data[sel]
+            indptr = np.concatenate(([0], np.cumsum(np.where(keep, lens, 0)))).astype(np.int64)
+        out.append((indptr, indices, data))
+    return out
 
 
 class _PackHandle:
@@ -339,7 +362,7 @@ class DevicePattern:
         torch = _torch()
         with torch.cuda.device(self.device):
             for k, t in self.host.items():
-                if k in _HOST_ONLY_ARRAYS:
+                if k in _HOST_ONLY_ARRAYS or (k in _POSTERIOR_ARRAYS and k not in self.dev):
                     continue
                 is_lazy = self._is_lazy(k)
                 if is_lazy != lazy and not (self.full and not lazy):
@@ -360,6 +383,19 @@ class DevicePattern:
         if self.tiled is not None:
             return True
         return k in _LAZY_ARRAYS and not (k == "rowptr" and self._need_rowptr)
+
+    def ensure_arrays(self, names):
+        """Make the named packed arrays resident (each is uploaded once; the descriptor is rebuilt if any was missing)."""
+        torch = _torch()
+        missing = [k for k in names if k not in self.dev]
+        if not missing:
+            return
+        with torch.cuda.device(self.device):
+            for k in missing:
+                t = self.host[k]
+                self.dev[k] = torch.zeros(16, dtype=torch.uint8, device=self.device) if t.numel() == 0 else t.to(self.device)
+                self.h2d_bytes += t.numel()
+        self._build_descriptor()
 
     def _weights_len(self, model1: bool) -> int:
         """Slots of the E-step weight vector: one per class (model 4), pair (2) or (class, gene) run (3); model 1 keeps
@@ -524,6 +560,58 @@ class DevicePattern:
     def acc_HT(self) -> np.ndarray:
         return self._fetch_T8(self.acc)
 
+    def copy_theta(self, previous: bool):
+        """Device copy of the current theta (or, `previous`, of the one that entered the last update) into `post_theta`,
+        the source of the next posterior; queued on the stream, no synchronisation."""
+        if getattr(self, "post_theta", None) is None:
+            self.post_theta = _torch().empty((self.T, 8), dtype=_torch().float64, device=self.device)
+        _lib.check(self.lib.gbrs_em_copy_theta(C.byref(self.desc), int(previous), self.post_theta.data_ptr(), self.stream()))
+
+    def posterior(self, model: int, theta_src, indptr, indices, reduce=None):
+        """gbrs_em_posterior: P = theta_src[t][h] * W[idx(n,t,h)] on the output pattern `indptr[h]` / `indices[h]` (host CSC
+        arrays of N x T, one pair per haplotype) -> list of H host value arrays.  `theta_src`: device [T][8].  `reduce`:
+        a callable summing a device tensor over the ranks of a row-sharded run (every rank fills its own classes only);
+        it also receives the error flag, so that every rank raises together."""
+        torch = _torch()
+        i = self.info
+        need = ["class_id", "pairs"]
+        if model != 4 or self._need_rowptr:
+            need.append("rowptr")
+        if model != 4:
+            if not self.packed.has_genes:
+                raise _lib.GbrsError("Group information matrix is missing.")
+            need.append("runptr")
+        self.ensure_arrays(need)
+        N = int(self.packed.N)
+        H = self.H
+        nbytes = C.c_int64()
+        _lib.check(self.lib.gbrs_em_posterior_scratch_bytes(C.byref(self.desc), int(model), N, C.byref(nbytes)))
+        wide = any(a.dtype.itemsize == 8 for a in indices)
+        with torch.cuda.device(self.device):
+            scratch = torch.empty(int(nbytes.value), dtype=torch.uint8, device=self.device)
+            d_ptr = [torch.from_numpy(np.ascontiguousarray(a, dtype=np.int64)).to(self.device) for a in indptr]
+            d_idx = [torch.from_numpy(np.ascontiguousarray(a, dtype=np.int64 if wide else np.int32)).to(self.device)
+                     for a in indices]
+            vals = [torch.empty(max(int(a.shape[0]), 1), dtype=torch.float64, device=self.device) for a in indices]
+            P = C.c_void_p * H
+            rc = self.lib.gbrs_em_posterior(
+                C.byref(self.desc), int(model), C.c_void_p(theta_src.data_ptr()),
+                C.c_void_p(self.dev["class_id"].data_ptr()) if i["n_classes"] > 0 else None, N,
+                P(*[t.data_ptr() for t in d_ptr]), P(*[t.data_ptr() for t in d_idx]), 8 if wide else 4,
+                P(*[t.data_ptr() for t in vals]), C.c_void_p(scratch.data_ptr()), int(nbytes.value), self.stream())
+            if reduce is not None:  # every rank learns whether any rank failed before anyone raises
+                flag = torch.tensor([-rc], dtype=torch.int32, device=self.device)
+                reduce(flag, "max")
+                worst = -int(flag.item())
+                if worst != _lib.GBRS_OK and rc == _lib.GBRS_OK:
+                    raise FloatingPointError("non-finite posterior probability on another rank") \
+                        if worst == _lib.GBRS_E_NUMERIC else _lib.GbrsError("posterior failed on another rank")
+            _lib.check(rc)
+            if reduce is not None:
+                for v in vals:
+                    reduce(v, "sum")
+            return [v[: a.shape[0]].cpu().numpy() for v, a in zip(vals, indices)]
+
     def alignment_counts(self, gene_level=False, n_real_genes=0):
         torch = _torch()
         self.ensure_full(model=4)  # the run tables, not model 1's weight vector
@@ -574,6 +662,10 @@ class EMfactory:
         self._weighted = False
         self._gene_of = None
         self._counts_host = None
+        # what the reference's `probability` would hold after the last call (posterior_probability()): None before
+        # prepare(); ("incidence",) after reset(); ("weighted",) after prepare() of a matrix with stored values;
+        # ("theta", model) after an E-step / update, the source theta being the pattern's `post_theta` snapshot
+        self._post = None
         self.num_iters = 0
         self.err_history = np.zeros(0)
         self.rank, self.world = 0, 1
@@ -825,6 +917,8 @@ class EMfactory:
             self.target_lengths = self._read_lengths(lenfile, read_length)
         self._pattern = None
         self.reset(pseudocount)
+        if self._weighted:  # prepare() normalises the stored values; reset() replaces them by ones first
+            self._post = ("weighted",)
 
     def reset(self, pseudocount: float = 0.0) -> None:
         """EMfactory.reset (EMfactory.py:113-138): theta0 from the incidence pattern."""
@@ -844,6 +938,7 @@ class EMfactory:
         self._raise_on_ctrl_error(ctrl, "the initial expression estimate")
         self._fetch_theta()
         self._counts_host = None
+        self._post = ("incidence",)
         self.num_iters = 0
 
     def _weighted_theta0(self, pseudocount: float) -> np.ndarray:
@@ -891,6 +986,8 @@ class EMfactory:
 
             dist.all_reduce(pat.acc, op=dist.ReduceOp.SUM, group=self._group)
         self._counts_host = None
+        pat.copy_theta(previous=False)  # theta does not move: the posterior is the E-step of the current one
+        self._post = ("theta", int(model))
 
     def update_allelic_expression(self, model: int = 3) -> None:
         """A single EM step (EMfactory.py:214-232): E-step, then theta = numerator / effective length."""
@@ -908,6 +1005,16 @@ class EMfactory:
         self._raise_on_ctrl_error(ctrl)
         self._fetch_theta()
         self._counts_host = None
+        self._snapshot_posterior_source(pat, model, 1)
+
+    def _snapshot_posterior_source(self, pat, model, n_updates):
+        """After `n_updates` updates the posterior of the reference's `probability` is the E-step of the theta that
+        entered the last one.  The loop has flipped the ping-pong after it (updates queued past the stop are no-ops), so
+        that theta is the other half; it is copied before a later set_theta (e.g. after report_depths' in-place TPM
+        scaling) can overwrite it.  No update: the previous posterior stays."""
+        if n_updates > 0:
+            pat.copy_theta(previous=True)
+            self._post = ("theta", int(model))
 
     @staticmethod
     def _raise_on_ctrl_error(ctrl, what="the EM update"):
@@ -960,6 +1067,7 @@ class EMfactory:
         self.num_iters = n
         self._fetch_theta()
         self._counts_host = None
+        self._snapshot_posterior_source(pat, model, n)
 
     # ---------------------------------------------------------------------------------------------------------------
     # reports
@@ -1014,7 +1122,77 @@ class EMfactory:
                 self._theta_dirty = True
         self._write_report(filename, lname, depths, reorder, notes)
 
-    def export_posterior_probability(self, filename: str, title: str = "Posterior Probability") -> None:
+    def export_posterior_probability(self, filename: str, title: str = "Posterior Probability",
+                                     incidence_only: bool = True) -> None:
         """Writes the pattern + counts, exactly what the reference's default `incidence_only=True` save emits
-        (EMfactory.py:382-392, AlignmentPropertyMatrix.py:484)."""
-        self.probability.save(h5file=filename, title=title)
+        (EMfactory.py:382-392, AlignmentPropertyMatrix.py:484).  `incidence_only=False`: the values of
+        `posterior_probability()` as well (the reference's `probability.save(..., incidence_only=False)`)."""
+        if incidence_only:
+            self.probability.save(h5file=filename, title=title)
+        else:
+            self.posterior_probability().save(h5file=filename, title=title, incidence_only=False)
+
+    # ---------------------------------------------------------------------------------------------------------------
+    # posterior read-origin probabilities
+    # ---------------------------------------------------------------------------------------------------------------
+    def posterior_probability(self) -> APM:
+        """The posterior read-origin probabilities the reference's `probability` holds after the last call
+        (EMfactory.update_probability_at_read_level, EMfactory.py:146-212): a new AlignmentPropertyMatrix with the shape,
+        names, counts and groups of `probability` and, per haplotype, a float64 CSC in canonical form holding
+        P[n,t,h] on the EM's pattern (stored entries, minus the columns of a `locus_hapmask` restriction).
+          after prepare() / reset():            the stored values normalised per class (1 / entries of the class for
+                                                a pure incidence matrix; reset() sets the values to 1 first)
+          after update_probability_at_read_level(model):  the E-step of `model` from the current theta
+          after update_allelic_expression(model) / run(model, ...): the E-step of the theta that entered the last update
+        Row-sharded runs: every rank computes its own classes and the values are summed over the group, so every rank
+        returns the whole matrix (`shard="local"`: the posterior of the matrix this rank was given).  A class whose
+        normaliser is 0 raises FloatingPointError, as the reference does.  `probability` itself is not changed."""
+        from scipy.sparse import csc_matrix
+
+        if self._post is None:
+            raise RuntimeError("no posterior yet: call prepare() first")
+        p = self.probability
+        T, H, N = p.shape
+        pattern = posterior_pattern(p, self._hapmask)
+        if self._post[0] == "weighted":
+            values = self._weighted_posterior(pattern, N)
+        else:
+            torch = _torch()
+            pat = self._ensure_pattern()
+            if self._post[0] == "incidence":
+                model, theta_src = 4, torch.ones((T, 8), dtype=torch.float64, device=pat.device)
+            else:
+                model, theta_src = self._post[1], pat.post_theta
+            reduce = None
+            if self.world > 1 and not self._presharded:
+                import torch.distributed as dist
+
+                def reduce(t, op):
+                    dist.all_reduce(t, op=dist.ReduceOp.MAX if op == "max" else dist.ReduceOp.SUM, group=self._group)
+
+            values = pat.posterior(model, theta_src, [a[0] for a in pattern], [a[1] for a in pattern], reduce=reduce)
+        out = APM()
+        out.shape = p.shape
+        out.num_loci, out.num_haplotypes, out.num_reads = p.shape
+        out.finalized = True
+        out.count = None if p.count is None else np.array(p.count, copy=True)
+        out._copy_names(p)
+        out._copy_group_info(p)
+        out.data = [csc_matrix((values[h], np.array(pattern[h][1], copy=True), pattern[h][0]), shape=(N, T))
+                    for h in range(H)]
+        return out
+
+    @staticmethod
+    def _weighted_posterior(pattern, N):
+        """prepare()'s posterior of a matrix with stored values: normalize_reads(READ) of the values (host, like the
+        initial estimate computed from them)."""
+        rows = np.zeros(N)
+        for _, indices, data in pattern:
+            rows += np.bincount(indices, weights=data, minlength=N)
+        out = []
+        for _, indices, data in pattern:
+            den = rows[indices]
+            if np.any(den == 0.0):
+                raise FloatingPointError("a class whose stored values sum to 0 has no posterior (0 / 0)")
+            out.append(np.asarray(data, dtype=np.float64) / den)
+        return out

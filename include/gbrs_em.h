@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define GBRS_EM_ABI_VERSION 6
+#define GBRS_EM_ABI_VERSION 7
 #define GBRS_HPAD 8 /* haplotype slots per locus line */
 #define GBRS_KMAX 8 /* classes with up to this many (class, locus) pairs take the fixed-width row pass */
 #define GBRS_DEEP_LOCUS_ITEMS 8 /* a locus with more partial sums (column-pass items / tile slots) than this is summed by a
@@ -100,6 +100,7 @@ int gbrs_pack_get_info(gbrs_pack_t p, gbrs_pack_info* info);
  *   "rowptr"  uint32 [n_classes+1]   "pairs"   uint32 [n_pairs]  (locus | mask<<24, sorted by (gene, locus) in a class;
  *                                     class n < bucket_class0[GBRS_KMAX] with k pairs starts at bucket_pair0[k-1] + (n - bucket_class0[k-1]) * k)
  *   "count"   double [n_classes]     "runptr"  uint32 [n_classes+1]
+ *   "class_id" uint32 [n_classes]    input class id of every packed class (the inverse of the class order)
  *   "ent_cls" / "ent_pair" / "ent_run"  entry words [n_entries], locus-major (index | mask << (8*entry_bytes-8));
  *                                     padding words carry an empty mask and index n_classes / n_pairs / n_runs
  *   "item_off" uint32 [n_items+1]    "locus_item_ptr" uint32 [T+1]   "item_order" uint32 [n_items]
@@ -122,6 +123,7 @@ typedef struct {
   const uint32_t* pairs;       /* [n_pairs] */
   const double* count;         /* [n_classes] */
   const uint32_t* runptr;      /* [n_classes + 1] */
+  const uint32_t* class_id;    /* [n_classes] */
   const void* ent_cls;         /* [n_entries] entry words (entry_bytes each) */
   const void* ent_pair;
   const void* ent_run;
@@ -320,6 +322,26 @@ int gbrs_em_launch_estep(const gbrs_em_dev* d, int model, void* stream);
 /* Second half (after `acc` holds the sum over all shards): theta' = acc / efflen (EMfactory.py:228-232), TPM-scaled
  * isoform-total L1 change and the stop test (EMfactory.py:267-279), entirely on the device. */
 int gbrs_em_launch_update(const gbrs_em_dev* d, void* stream);
+
+/* Posterior read-origin probabilities P[n,t,h] of one E-step (EMfactory.update_probability_at_read_level,
+ * EMfactory.py:146-212: what the reference leaves in `probability`), written on a caller-supplied pattern.  For every
+ * model  count_n * P[n,t,h] = theta[t][h] * W[idx(n,t,h)]  with W the weight vector of the row pass (idx = class for
+ * model 4, (class, gene) run for model 3, pair for model 2, run * 8 + h for model 1), so the call runs the row pass of
+ * `model` on `theta_src` ([T][8], device) with unit counts into `scratch` and gathers theta_src[t][h] * W[idx] onto the
+ * output pattern: per haplotype h < H a CSC over (N input classes) x T, `indptr[h]` int64 [T+1] and `indices[h]`
+ * (`index_bytes` 4 or 8) device arrays, sorted indices.  Every entry must be a stored entry of the packed pattern (the
+ * incidence the descriptor was packed from, minus the -G restriction) or belong to a class outside this shard, which
+ * gets 0.  `class_id` is the packer's array of that name (device).  Nothing the EM owns is written: theta, acc, weights,
+ * subset / gene tables, iso, ctrl / scal / err_log and the exchange buffers stay as they are.  `scratch` (device, 256-byte
+ * aligned) holds at least gbrs_em_posterior_scratch_bytes(d, model, N) bytes.  Synchronises the stream; GBRS_E_NUMERIC
+ * if a class has a zero normaliser or a value is not finite (the reference raises FloatingPointError). */
+int gbrs_em_posterior_scratch_bytes(const gbrs_em_dev* d, int model, int64_t N, int64_t* bytes);
+int gbrs_em_posterior(const gbrs_em_dev* d, int model, const double* theta_src, const uint32_t* class_id, int64_t N,
+                      const int64_t* const* indptr, const void* const* indices, int32_t index_bytes,
+                      double* const* values, void* scratch, int64_t scratch_bytes, void* stream);
+/* Device-to-device copy of the current theta (previous = 0) or of the other half of the ping-pong (previous = 1: after
+ * an update, the theta that entered it) into dst [T][8]; the parity is read on the device, nothing synchronises. */
+int gbrs_em_copy_theta(const gbrs_em_dev* d, int previous, double* dst, void* stream);
 
 /* Per-kernel device timing of the first half (CUDA events on `stream` around the row pass, the column pass and the
  * numerator kernel), used by bench.py for the roofline figure.  gbrs_prof_read synchronises, returns the summed
