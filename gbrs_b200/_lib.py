@@ -15,7 +15,7 @@ LIB_PATH = os.environ.get("GBRS_LIB_PATH") or os.path.join(HERE, "_C", "libgbrs_
 GBRS_HPAD = 8
 GBRS_KMAX = 8
 GBRS_PART_SLOTS = 4096
-ABI_VERSION = 7
+ABI_VERSION = 8
 CTRL_ITERS, CTRL_DONE, CTRL_ERROR, CTRL_PARITY, CTRL_MAX_ITERS, CTRL_PREPARED = range(6)
 SCAL_ERR, SCAL_SUM_PREV, SCAL_TARGET, SCAL_SUM_CUR = range(4)
 
@@ -94,7 +94,8 @@ class EmDev(C.Structure):
                 ("tile_max_a_bytes", C.c_int32), ("tile_max_b_bytes", C.c_int32), ("tile_n_deep_loci", C.c_int32),
                 ("theta", C.c_void_p), ("efflen", C.c_void_p), ("acc", C.c_void_p), ("iso", C.c_void_p),
                 ("weights", C.c_void_p), ("subsets", C.c_void_p), ("wit", C.c_void_p), ("part", C.c_void_p), ("gene_hap", C.c_void_p),
-                ("gamma", C.c_void_p), ("err_log", C.c_void_p), ("scal", C.c_void_p), ("ctrl", C.c_void_p)]
+                ("gamma", C.c_void_p), ("err_log", C.c_void_p), ("scal", C.c_void_p), ("ctrl", C.c_void_p),
+                ("zero_count_absent", C.c_int32), ("reserved", C.c_int32)]
 
 
 POLL_CB = C.CFUNCTYPE(None, C.c_int32, C.c_int32, C.POINTER(C.c_double), C.c_void_p)
@@ -142,6 +143,10 @@ SYMBOLS = {
                                     C.POINTER(C.c_void_p), C.c_int32, C.POINTER(C.c_void_p), C.c_void_p, C.c_int64,
                                     C.c_void_p]),
     "gbrs_em_copy_theta": (C.c_int, [C.POINTER(EmDev), C.c_int, C.c_void_p, C.c_void_p]),
+    "gbrs_boot_scratch_bytes": (C.c_int, [C.c_int64, C.POINTER(C.c_int64)]),
+    "gbrs_boot_guide": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    "gbrs_boot_resample": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_int64,
+                                     C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "gbrs_write_table": (C.c_int, [C.c_char_p, C.c_char_p, C.POINTER(C.c_char_p), C.c_int64, C.c_void_p, C.c_int32,
                                    C.POINTER(C.c_char_p), C.c_void_p, C.c_int32]),
     "gbrs_parse_lengths": (C.c_int, [C.c_char_p, C.POINTER(C.c_char_p), C.c_int64, C.POINTER(C.c_char_p), C.c_int32,

@@ -38,6 +38,8 @@ def quantify(
     tolerance: Annotated[float, typer.Option("-t", "--tolerance", help="tolerance for EM termination (default: 0.0001 in TPM)")] = 0.0001,
     report_alignment_counts: Annotated[bool, typer.Option("-a", "--report-alignment-counts", help="whether to report alignment counts")] = False,
     report_posterior: Annotated[bool, typer.Option("-w", "--report-posterior", help="whether to report posterior probabilities")] = False,
+    bootstrap: Annotated[int, typer.Option("--bootstrap", help="bootstrap replicates, written to <outbase>.bootstrap.npz after the reports (default: 0 = none)")] = 0,
+    bootstrap_seed: Annotated[int, typer.Option("--bootstrap-seed", help="seed of the bootstrap replicates (default: 0)")] = 0,
     verbose: Annotated[int, typer.Option("-v", "--verbose", count=True, help="specify multiple times for more verbose output")] = 0,
 ) -> None:
     logger = utils.configure_logging("gbrs", verbose)
@@ -51,7 +53,8 @@ def quantify(
             length_file=str(length_file) if length_file else None,
             genotype_file=str(genotype_file) if genotype_file else None,
             outbase=outbase, multiread_model=multiread_model, pseudocount=pseudocount, max_iters=max_iters,
-            tolerance=tolerance, report_alignment_counts=report_alignment_counts, report_posterior=report_posterior)
+            tolerance=tolerance, report_alignment_counts=report_alignment_counts, report_posterior=report_posterior,
+            bootstrap=bootstrap, bootstrap_seed=bootstrap_seed)
     except Exception as e:  # reference policy: log and return
         if logger.level == logging.DEBUG:
             logger.exception(e)
@@ -147,6 +150,8 @@ def run(
     tolerance: Annotated[float, typer.Option("-t", "--tolerance", help="tolerance for EM termination (default: 0.0001 in TPM)")] = 0.0001,
     report_alignment_counts: Annotated[bool, typer.Option("-c", "--report-alignment-counts", help="whether to report alignment counts")] = False,
     report_posterior: Annotated[bool, typer.Option("-w", "--report-posterior", help="whether to report posterior probabilities")] = False,
+    bootstrap: Annotated[int, typer.Option("--bootstrap", help="bootstrap replicates, written to <outbase>.bootstrap.npz after the reports (default: 0 = none)")] = 0,
+    bootstrap_seed: Annotated[int, typer.Option("--bootstrap-seed", help="seed of the bootstrap replicates (default: 0)")] = 0,
     verbose: Annotated[int, typer.Option("-v", "--verbose", count=True, help="specify multiple times for more verbose output")] = 0,
 ) -> None:
     """Flag surface of the reference's `emase run` (/root/reference/src/gbrs/emase/commands.py:315-356)."""
@@ -159,7 +164,8 @@ def run(
             alignment_file=str(alignment_file), group_file=str(group_file) if group_file else None,
             length_file=str(length_file) if length_file else None, outbase=outbase, multiread_model=multiread_model,
             read_length=read_length, pseudocount=pseudocount, max_iters=max_iters, tolerance=tolerance,
-            report_alignment_counts=report_alignment_counts, report_posterior=report_posterior)
+            report_alignment_counts=report_alignment_counts, report_posterior=report_posterior,
+            bootstrap=bootstrap, bootstrap_seed=bootstrap_seed)
     except Exception as e:
         if logger.level == logging.DEBUG:
             logger.exception(e)

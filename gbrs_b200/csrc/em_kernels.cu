@@ -394,7 +394,7 @@ struct RowPlan {                     // host-computed: work units ordered from t
   int64_t unit_end[GBRS_KMAX];       // unit_end[i] = one past the last unit (= 32 * unr classes) of width GBRS_KMAX - i
 };
 
-template <int K, bool UNIT>
+template <int K, bool UNIT, bool ZA>
 __device__ __forceinline__ void row_classes_m4(const gbrs_em_dev& d, int64_t class0, int64_t class_end,
                                                int64_t bucket_class0, int64_t bucket_pair0) {
   constexpr int UNR = unr_of(K);
@@ -440,7 +440,7 @@ __device__ __forceinline__ void row_classes_m4(const gbrs_em_dev& d, int64_t cla
   }
 #pragma unroll
   for (int u = 0; u < UNR; ++u)
-    if (n[u] < class_end) d.weights[n[u]] = fast_div(cnt[u], s[u]);
+    if (n[u] < class_end) d.weights[n[u]] = (ZA && cnt[u] == 0.0) ? 0.0 : fast_div(cnt[u], s[u]);
 }
 
 // One launch per width range [KLO, KHI]: the narrow classes (four out of five have at most three pairs) are not compiled for
@@ -448,7 +448,10 @@ __device__ __forceinline__ void row_classes_m4(const gbrs_em_dev& d, int64_t cla
 #ifndef GBRS_ROW_MINBLOCKS
 #define GBRS_ROW_MINBLOCKS 1  // resident blocks per SM the model-4 row pass is compiled for (1: no register cap)
 #endif
-template <bool UNIT, int KLO, int KHI>
+// ZA (descriptor flag zero_count_absent): a class of count 0 is absent -- weight 0 without a division, so a class whose
+// entries all have theta 0 does not turn into 0 / 0 (bootstrap replicates drop classes).  The default instantiation
+// (ZA = false) is the row pass of every ordinary update, unchanged.
+template <bool UNIT, int KLO, int KHI, bool ZA = false>
 __global__ void __launch_bounds__(kThreads, GBRS_ROW_MINBLOCKS) k_weights_m4(const __grid_constant__ gbrs_em_dev d,
                                                           const __grid_constant__ RowPlan plan) {
   if (!UNIT && d.ctrl[GBRS_CTRL_DONE]) return;
@@ -467,7 +470,7 @@ __global__ void __launch_bounds__(kThreads, GBRS_ROW_MINBLOCKS) k_weights_m4(con
     const int64_t class0 = c0 + (u - unit0) * cpu;
 #define GBRS_ROW_CASE(K) \
   case K:                \
-    if constexpr (K >= KLO && K <= KHI) row_classes_m4<K, UNIT>(d, class0, c1, c0, p0); \
+    if constexpr (K >= KLO && K <= KHI) row_classes_m4<K, UNIT, ZA>(d, class0, c1, c0, p0); \
     break;
     switch (k) {
       GBRS_ROW_CASE(1) GBRS_ROW_CASE(2) GBRS_ROW_CASE(3) GBRS_ROW_CASE(4)
@@ -479,7 +482,7 @@ __global__ void __launch_bounds__(kThreads, GBRS_ROW_MINBLOCKS) k_weights_m4(con
 }
 
 // Classes with more than GBRS_KMAX pairs: one thread per class over the CSR row.
-template <bool UNIT>
+template <bool UNIT, bool ZA = false>
 __global__ void __launch_bounds__(kThreads) k_weights_m4_long(const gbrs_em_dev d) {
   if (!UNIT && d.ctrl[GBRS_CTRL_DONE]) return;
   const int64_t stride = (int64_t) gridDim.x * blockDim.x;
@@ -491,7 +494,8 @@ __global__ void __launch_bounds__(kThreads) k_weights_m4_long(const gbrs_em_dev 
       if (UNIT) s += (double) __popc(w >> 24);
       else s += pair_sum(d.subsets, w);
     }
-    d.weights[n] = __ldg(d.count + n) / s;
+    const double c = __ldg(d.count + n);
+    d.weights[n] = (ZA && c == 0.0) ? 0.0 : c / s;
   }
 }
 
@@ -2182,7 +2186,7 @@ int launch_exchange(const gbrs_em_dev* d, cudaStream_t s) {
   return GBRS_OK;
 }
 
-template <bool UNIT, int KLO, int KHI>
+template <bool UNIT, int KLO, int KHI, bool ZA>
 int launch_row_m4_range(const gbrs_em_dev* d, cudaStream_t s) {
   RowPlan plan;
   int64_t units = 0;
@@ -2194,21 +2198,21 @@ int launch_row_m4_range(const gbrs_em_dev* d, cudaStream_t s) {
     plan.unit_end[i] = units;
   }
   if (units > 0) {
-    k_weights_m4<UNIT, KLO, KHI><<<resident_grid(k_weights_m4<UNIT, KLO, KHI>, units * 32), kThreads, 0, s>>>(*d, plan);
+    k_weights_m4<UNIT, KLO, KHI, ZA><<<resident_grid(k_weights_m4<UNIT, KLO, KHI, ZA>, units * 32), kThreads, 0, s>>>(*d, plan);
     GBRS_LAUNCH_CHECK("k_weights_m4");
   }
   return GBRS_OK;
 }
 
-template <bool UNIT>
+template <bool UNIT, bool ZA = false>
 int launch_row_m4(const gbrs_em_dev* d, cudaStream_t s) {
   // one launch for all widths: here the narrow classes set the register budget (four classes per thread), so a split by
   // width buys no occupancy and would cost a launch gap (models 2-3 do split: their wide classes need 64-98 registers)
-  if (int rc = launch_row_m4_range<UNIT, 1, GBRS_KMAX>(d, s)) return rc;
+  if (int rc = launch_row_m4_range<UNIT, 1, GBRS_KMAX, ZA>(d, s)) return rc;
   const int64_t n_long = d->n_classes - d->bucket_class0[GBRS_KMAX];
   if (n_long > 0) {
     if (!d->rowptr) { gbrs_set_error("row pass: classes wider than GBRS_KMAX need rowptr"); return GBRS_E_ARG; }
-    k_weights_m4_long<UNIT><<<grid_for(n_long), kThreads, 0, s>>>(*d);
+    k_weights_m4_long<UNIT, ZA><<<grid_for(n_long), kThreads, 0, s>>>(*d);
     GBRS_LAUNCH_CHECK("k_weights_m4_long");
   }
   return GBRS_OK;
@@ -2276,7 +2280,11 @@ inline gbrs_em_dev locus_view(const gbrs_em_dev* d, bool tiles) {
 // gene totals too (k_gene_totals before this).
 int launch_row_pass(const gbrs_em_dev* d, int model, cudaStream_t s) {
   switch (model) {
-    case 4: if (int rc4 = launch_row_m4<false>(d, s)) return rc4; break;
+    case 4: {
+      const int rc4 = d->zero_count_absent ? launch_row_m4<false, true>(d, s) : launch_row_m4<false>(d, s);
+      if (rc4) return rc4;
+      break;
+    }
     case 3:
     case 2: {
       const int64_t n_fixed = d->bucket_class0[GBRS_KMAX], n_long = d->n_classes - n_fixed;
@@ -2466,6 +2474,133 @@ __global__ void __launch_bounds__(kThreads) k_copy_theta(const gbrs_em_dev d, in
   const int64_t total = (int64_t) d.T * GBRS_HPAD;
   const int64_t stride = (int64_t) gridDim.x * blockDim.x;
   for (int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) dst[i] = src[i];
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Bootstrap resampler (gbrs_boot_guide / gbrs_boot_resample; the contract is in include/gbrs_em.h).  Draws come from
+// Philox4x32-10 (Salmon et al., SC'11; the constants of Random123 and of curand), written out here so that the host SIMT
+// shim compiles it as it is.  A draw u is read floor(u * M / 2^64), the high half of the product; its class is an upper bound on the
+// int64 prefix of the counts.  A plain binary search over the whole prefix (40 MB at C2) is a chain of ~23 dependent
+// gathers per draw; the guide table cuts it to the few classes between two guide entries: with G = 2^bits entries,
+// entry g = class of read floor(g * M / G) = class of the draw g << (64 - bits), and a draw u lies between entries
+// u >> (64 - bits) and the next one (both readings are monotone in u).
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int kBootGuideBitsMax = 24;
+
+// high halves of the 32 x 32 and 64 x 64-bit products: the hardware intrinsics on the device, the same arithmetic in
+// portable C++ where the kernels are compiled for the host (__CUDA_ARCH__ undefined)
+__device__ __forceinline__ uint32_t mul32hi(uint32_t a, uint32_t b) {
+#ifdef __CUDA_ARCH__
+  return __umulhi(a, b);
+#else
+  return (uint32_t) (((uint64_t) a * b) >> 32);
+#endif
+}
+
+__device__ __forceinline__ uint64_t mul64hi(uint64_t a, uint64_t b) {
+#ifdef __CUDA_ARCH__
+  return __umul64hi(a, b);
+#else
+  return (uint64_t) (((unsigned __int128) a * b) >> 64);
+#endif
+}
+
+__device__ __forceinline__ void philox4x32_10(uint32_t (&x)[4], uint32_t k0, uint32_t k1) {
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    const uint32_t hi0 = mul32hi(0xD2511F53u, x[0]), lo0 = 0xD2511F53u * x[0];
+    const uint32_t hi1 = mul32hi(0xCD9E8D57u, x[2]), lo1 = 0xCD9E8D57u * x[2];
+    const uint32_t y0 = hi1 ^ x[1] ^ k0, y2 = hi0 ^ x[3] ^ k1;
+    x[0] = y0;
+    x[1] = lo1;
+    x[2] = y2;
+    x[3] = lo0;
+    k0 += 0x9E3779B9u;  // key schedule (the bump after the last round is never used)
+    k1 += 0xBB67AE85u;
+  }
+}
+
+// first class n in [lo, hi] with P[n] > k (the caller guarantees P[hi] > k)
+__device__ __forceinline__ int64_t boot_upper_bound(const int64_t* __restrict__ P, int64_t lo, int64_t hi, int64_t k) {
+  while (lo < hi) {
+    const int64_t mid = lo + ((hi - lo) >> 1);
+    if (__ldg(P + mid) > k) hi = mid;
+    else lo = mid + 1;
+  }
+  return lo;
+}
+
+__global__ void __launch_bounds__(kThreads) k_boot_guide(const int64_t* __restrict__ P, int64_t N, uint64_t M, int bits,
+                                                         uint32_t* __restrict__ guide) {
+  const int64_t G = int64_t(1) << bits, stride = (int64_t) gridDim.x * blockDim.x;
+  for (int64_t g = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; g <= G; g += stride) {
+    int64_t c = N - 1;  // entry G: past every read
+    if (g < G) {
+      const uint64_t u = bits ? (uint64_t) g << (64 - bits) : 0ull;
+      c = boot_upper_bound(P, 0, N - 1, (int64_t) mul64hi(u, M));
+    }
+    guide[g] = (uint32_t) c;
+  }
+}
+
+// one thread per draw pair (grid-stride): Philox, the two reads, their classes, one integer atomic per draw
+__global__ void __launch_bounds__(kThreads) k_boot_sample(const int64_t* __restrict__ P, uint64_t M, int bits,
+                                                          const uint32_t* __restrict__ guide, uint64_t seed, uint32_t rep,
+                                                          unsigned long long* __restrict__ hist) {
+  const uint64_t n_pairs = (M + 1) >> 1, stride = (uint64_t) gridDim.x * blockDim.x;
+  const uint32_t k0 = (uint32_t) seed, k1 = (uint32_t) (seed >> 32);
+  for (uint64_t j = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; j < n_pairs; j += stride) {
+    uint32_t x[4] = {(uint32_t) j, (uint32_t) (j >> 32), rep, 0u};
+    philox4x32_10(x, k0, k1);
+    const uint64_t u[2] = {(uint64_t) x[0] | ((uint64_t) x[1] << 32), (uint64_t) x[2] | ((uint64_t) x[3] << 32)};
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+      if (2 * j + q >= M) break;  // odd M: the second draw of the last pair is unused
+      const int64_t k = (int64_t) mul64hi(u[q], M);
+      const uint64_t g = bits ? u[q] >> (64 - bits) : 0ull;
+      const int64_t n = boot_upper_bound(P, __ldg(guide + g), __ldg(guide + g + 1), k);
+      atomicAdd(hist + n, 1ull);
+    }
+  }
+}
+
+// replicate counts in packed class order
+__global__ void __launch_bounds__(kThreads) k_boot_scatter(const unsigned long long* __restrict__ hist,
+                                                           const uint32_t* __restrict__ class_id, int64_t n_classes,
+                                                           double* __restrict__ count) {
+  const int64_t stride = (int64_t) gridDim.x * blockDim.x;
+  for (int64_t p = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; p < n_classes; p += stride)
+    count[p] = (double) hist[__ldg(class_id + p)];
+}
+
+inline int boot_bits(int64_t N) {
+  int b = 0;
+  while (b < kBootGuideBitsMax && (int64_t(1) << b) < N) ++b;
+  return b;
+}
+
+// scratch of the resampler: histogram uint64 [N] | guide uint32 [G + 1] (each 256-byte aligned)
+struct BootScratch {
+  int64_t hist, guide, total;
+};
+inline BootScratch boot_scratch(int64_t N) {
+  auto up = [](int64_t b) { return (b + 255) & ~int64_t(255); };
+  BootScratch L;
+  L.hist = 0;
+  L.guide = up(N * (int64_t) sizeof(unsigned long long));
+  L.total = L.guide + up(((int64_t(1) << boot_bits(N)) + 1) * (int64_t) sizeof(uint32_t));
+  return L;
+}
+
+int check_boot(const int64_t* prefix, int64_t N, int64_t M, void* scratch, int64_t scratch_bytes, const char* who) {
+  if (!prefix || !scratch || N < 1 || N >= (int64_t(1) << 32) || M < 1 || M > (int64_t(1) << 53)) {
+    gbrs_set_error(std::string(who) + ": bad argument (1 <= N < 2^32 classes and 1 <= M <= 2^53 reads)");
+    return GBRS_E_ARG;
+  }
+  if (scratch_bytes < boot_scratch(N).total) { gbrs_set_error(std::string(who) + ": scratch too small"); return GBRS_E_ARG; }
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) { gbrs_set_error(std::string(who) + ": no CUDA device (there is no CPU fallback)"); return GBRS_E_CUDA; }
+  return GBRS_OK;
 }
 
 }  // namespace
@@ -2970,5 +3105,45 @@ extern "C" int gbrs_em_copy_theta(const gbrs_em_dev* d, int previous, double* ds
   if (!dst || (previous != 0 && previous != 1)) { gbrs_set_error("gbrs_em_copy_theta: bad argument"); return GBRS_E_ARG; }
   k_copy_theta<<<grid_for((int64_t) d->T * GBRS_HPAD), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(*d, previous, dst);
   GBRS_LAUNCH_CHECK("k_copy_theta");
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_boot_scratch_bytes(int64_t N, int64_t* bytes) {
+  if (!bytes || N < 1) { gbrs_set_error("gbrs_boot_scratch_bytes: bad argument"); return GBRS_E_ARG; }
+  *bytes = boot_scratch(N).total;
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_boot_guide(const int64_t* prefix, int64_t N, int64_t M, void* scratch, int64_t scratch_bytes, void* stream) {
+  if (int rc = check_boot(prefix, N, M, scratch, scratch_bytes, "gbrs_boot_guide")) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int bits = boot_bits(N);
+  uint32_t* guide = reinterpret_cast<uint32_t*>(static_cast<char*>(scratch) + boot_scratch(N).guide);
+  k_boot_guide<<<grid_for((int64_t(1) << bits) + 1), kThreads, 0, s>>>(prefix, N, (uint64_t) M, bits, guide);
+  GBRS_LAUNCH_CHECK("k_boot_guide");
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_boot_resample(const int64_t* prefix, int64_t N, int64_t M, uint64_t seed, uint32_t replicate,
+                                  const uint32_t* class_id, int64_t n_classes, void* scratch, int64_t scratch_bytes,
+                                  double* count_out, void* stream) {
+  if (int rc = check_boot(prefix, N, M, scratch, scratch_bytes, "gbrs_boot_resample")) return rc;
+  if (n_classes < 0 || n_classes > N || (n_classes > 0 && (!class_id || !count_out))) {
+    gbrs_set_error("gbrs_boot_resample: bad packed class arguments"); return GBRS_E_ARG;
+  }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const BootScratch L = boot_scratch(N);
+  char* base = static_cast<char*>(scratch);
+  unsigned long long* hist = reinterpret_cast<unsigned long long*>(base + L.hist);
+  const uint32_t* guide = reinterpret_cast<const uint32_t*>(base + L.guide);
+  GBRS_CUDA(cudaMemsetAsync(hist, 0, sizeof(unsigned long long) * (size_t) N, s));
+  const int64_t n_pairs = (M + 1) >> 1;
+  k_boot_sample<<<resident_grid(k_boot_sample, n_pairs), kThreads, 0, s>>>(prefix, (uint64_t) M, boot_bits(N), guide, seed,
+                                                                            replicate, hist);
+  GBRS_LAUNCH_CHECK("k_boot_sample");
+  if (n_classes > 0) {
+    k_boot_scatter<<<grid_for(n_classes), kThreads, 0, s>>>(hist, class_id, n_classes, count_out);
+    GBRS_LAUNCH_CHECK("k_boot_scatter");
+  }
   return GBRS_OK;
 }

@@ -19,13 +19,14 @@ Differences from the reference that a caller can observe (DESIGN.md section 6):
 """
 from __future__ import annotations
 
+import copy
 import ctypes as C
 import os
 import time
 
 import numpy as np
 
-from . import _lib, utils
+from . import _lib, bootstrap as _boot, utils
 from .apm import AlignmentPropertyMatrix as APM
 
 logger = utils.get_logger("gbrs")
@@ -612,6 +613,28 @@ class DevicePattern:
                     reduce(v, "sum")
             return [v[: a.shape[0]].cpu().numpy() for v, a in zip(vals, indices)]
 
+    def replicate_state(self, model: int):
+        """A second state set over the same packed arrays, for bootstrap replicates: its own theta ping-pong, numerator,
+        isoform totals, subset / weight / partial-sum / gene tables, control block and error log, and a count buffer at
+        a fixed address (the captured loop of gbrs_em_run_cb is keyed by the descriptor, so one graph serves every
+        replicate).  Lengths are shared.  Always the two-pass kernels (the tile blob holds its own copy of the counts), and
+        the model-4 row pass treats a class of count 0 as absent.  Nothing of this pattern's own state is touched."""
+        torch = _torch()
+        self.ensure_full(model=4)  # every array of the two-pass kernels resident (a tiled pattern has them lazy)
+        st = copy.copy(self)
+        st.tiled, st.desc, st._stage = None, None, None
+        st.dev = dict(self.dev)
+        st._alloc_state()
+        st.efflen = self.efflen
+        if model == 1:
+            st.weights = torch.zeros(st._weights_len(True), dtype=torch.float64, device=self.device)
+        st.count = torch.zeros(max(self.info["n_classes"], 1), dtype=torch.float64, device=self.device)
+        st.dev["count"] = st.count
+        st._build_descriptor()
+        st.desc.n_ranks = 1
+        st.desc.zero_count_absent = 1
+        return st
+
     def alignment_counts(self, gene_level=False, n_real_genes=0):
         torch = _torch()
         self.ensure_full(model=4)  # the run tables, not model 1's weight vector
@@ -1068,6 +1091,77 @@ class EMfactory:
         self._fetch_theta()
         self._counts_host = None
         self._snapshot_posterior_source(pat, model, n)
+
+    # ---------------------------------------------------------------------------------------------------------------
+    # bootstrap replicates
+    # ---------------------------------------------------------------------------------------------------------------
+    def bootstrap(self, replicates, model: int = 4, seed: int = 0, pseudocount: float = 0.0, tol: float = 0.0001,
+                  max_iters: int = 999) -> _boot.BootstrapResult:
+        """Bootstrap replicates of the estimates (DESIGN.md section 7.2).  `replicates`: an int n (= range(n)) or a
+        sequence of replicate indices (uint32).  Replicate r of `seed` resamples the M = sum(count) reads of the input
+        with replacement on the device (a pure function of seed, r and the counts: a subset of indices run alone gives
+        the same bits as in a larger call, on any packer or layout) and is then prepare(pseudocount) + run(model, tol,
+        max_iters) on the resampled counts, with the lengths, groups and -G restriction of this factory; classes drawn 0
+        times are absent, exactly as if the resampled reads had been compressed again.  Needs prepare() first.  The
+        replicates run on their own device state: everything this factory reports afterwards is bit-identical to before.
+        Refused (before any device work): row-sharded factories, weighted files, counts that are not non-negative
+        integers or sum to more than 2^53, M = 0."""
+        if model not in (1, 2, 3, 4):
+            raise RuntimeError("The read normalization model should be 1, 2, 3, or 4.")
+        if max_iters > ERR_LOG_CAP:
+            raise ValueError(f"max_iters above {ERR_LOG_CAP} is not supported")
+        if self.world > 1 or self._presharded:
+            raise NotImplementedError("bootstrap replicates of a row-sharded factory are not supported")
+        if self._pattern is None or self._post is None:
+            raise RuntimeError("bootstrap needs prepare() first")
+        if self._weighted:
+            raise NotImplementedError("bootstrap replicates of a weighted alignment file (stored values other than 1) "
+                                      "are not supported")
+        p = self.probability
+        T, H, N = p.shape
+        if model != 4 and p.num_groups == 0:
+            raise _lib.GbrsError("Group information matrix is missing.")
+        reps = _boot.replicate_indices(replicates)
+        counts = _boot.read_counts_of(p.count, N)
+        M = int(counts.sum())
+        if M == 0:
+            raise ValueError("bootstrap needs at least one read (the counts sum to 0)")
+        if not 0 <= int(seed) < 2 ** 64:
+            raise ValueError("the bootstrap seed must fit 64 bits")
+        torch = _torch()
+        pat = self._pattern
+        pat.ensure_arrays(["class_id"])
+        st = pat.replicate_state(model)
+        B, n_cls = int(reps.shape[0]), int(pat.info["n_classes"])
+        lib = pat.lib
+        with torch.cuda.device(pat.device):
+            prefix = torch.from_numpy(np.cumsum(counts)).to(pat.device)
+            nbytes = C.c_int64()
+            _lib.check(lib.gbrs_boot_scratch_bytes(N, C.byref(nbytes)))
+            scratch = torch.empty(int(nbytes.value), dtype=torch.uint8, device=pat.device)
+            _lib.check(lib.gbrs_boot_guide(C.c_void_p(prefix.data_ptr()), N, M, C.c_void_p(scratch.data_ptr()),
+                                           int(nbytes.value), pat.stream()))
+            theta_all = torch.empty((B, T, 8), dtype=torch.float64, device=pat.device)
+            acc_all = torch.empty((B, T, 8), dtype=torch.float64, device=pat.device)
+            iters = np.zeros(B, dtype=np.int64)
+            errs = np.zeros(max(max_iters, 1), dtype=np.float64)
+            class_id = C.c_void_p(pat.dev["class_id"].data_ptr()) if n_cls > 0 else None
+            for b, r in enumerate(reps.tolist()):
+                _lib.check(lib.gbrs_boot_resample(C.c_void_p(prefix.data_ptr()), N, M, int(seed), int(r), class_id, n_cls,
+                                                  C.c_void_p(scratch.data_ptr()), int(nbytes.value),
+                                                  C.c_void_p(st.count.data_ptr()), pat.stream()))
+                _lib.check(lib.gbrs_em_prepare_local(C.byref(st.desc), pat.stream()))
+                _lib.check(lib.gbrs_em_prepare_finish(C.byref(st.desc), float(pseudocount), pat.stream()))
+                n = C.c_int32(0)
+                _lib.check(lib.gbrs_em_run_cb(C.byref(st.desc), int(model), float(tol), int(max_iters),
+                                              int(self._poll_every), pat.stream(), C.byref(n), errs.ctypes.data, None, None))
+                iters[b] = n.value
+                _lib.check(lib.gbrs_em_copy_theta(C.byref(st.desc), 0, C.c_void_p(theta_all[b].data_ptr()), pat.stream()))
+                acc_all[b].copy_(st.acc)
+            theta = theta_all[:, :, :H].permute(0, 2, 1).contiguous().cpu().numpy()
+            acc = acc_all[:, :, :H].permute(0, 2, 1).contiguous().cpu().numpy()
+        return _boot.BootstrapResult(reps, int(seed), model, M, iters, theta, acc, grp_conv_mat=self.grp_conv_mat,
+                                     lname=p.lname, hname=p.hname, gname=p.gname if p.num_groups > 0 else None)
 
     # ---------------------------------------------------------------------------------------------------------------
     # reports

@@ -90,12 +90,25 @@ def _write_reports(em_factory, outbase, alignment_file, group_file, report_group
                                            pattern=unmasked_pattern)
 
 
+def _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters):
+    """`--bootstrap N`: N replicates (indices 0..N-1 of `bootstrap_seed`) after the point-estimate reports, written to
+    {outbase}.bootstrap.npz (BootstrapResult.save)."""
+    if bootstrap <= 0:
+        return
+    path = f"{outbase}.bootstrap.npz"
+    logger.info(f"Running {bootstrap} bootstrap replicates (seed {bootstrap_seed}): {path}")
+    res = em_factory.bootstrap(bootstrap, model=multiread_model, seed=bootstrap_seed, pseudocount=pseudocount,
+                               tol=tolerance, max_iters=max_iters)
+    res.save(path)
+
+
 def run(alignment_file: str, group_file: str = None, length_file: str = None, outbase: str = "emase",
         multiread_model: int = 4, read_length: int = 100, pseudocount: float = 0.0, max_iters: int = 999,
         tolerance: float = 0.0001, report_alignment_counts: bool = False, report_posterior: bool = False,
-        device=None, group=None) -> None:
+        device=None, group=None, bootstrap: int = 0, bootstrap_seed: int = 0) -> None:
     """`emase run` workflow (reference `gbrs.emase.emase_utils.run`, emase/emase_utils.py:594-696): the same EM without
-    the genotype restriction, with an explicit read length and no default group / length files."""
+    the genotype restriction, with an explicit read length and no default group / length files.  `bootstrap` /
+    `bootstrap_seed`: replicates written after the reports (see `_write_bootstrap`; 0 = none)."""
     report_group_counts = group_file is not None
     logger.info(f"Alignment File: {alignment_file}")
     logger.info(f"Group File: {group_file}")
@@ -113,15 +126,17 @@ def run(alignment_file: str, group_file: str = None, length_file: str = None, ou
         reuse_pattern = em_factory.world == 1 and em_factory._pattern.packed.has_genes
         _write_reports(em_factory, outbase, alignment_file, group_file, report_group_counts, report_alignment_counts,
                        report_posterior, unmasked=aln_mat, unmasked_pattern=em_factory._pattern if reuse_pattern else None)
+        _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters)
     logger.debug("Done")
 
 
 def quantify(alignment_file: str, group_file: str = None, length_file: str = None, genotype_file: str = None,
              outbase: str = "gbrs.quantified", multiread_model: int = 4, pseudocount: float = 0.0,
              max_iters: int = 999, tolerance: float = 0.0001, report_alignment_counts: bool = False,
-             report_posterior: bool = False, device=None, group=None) -> None:
-    """Quantify expected read counts.  `device` / `group` are the only additions: the CUDA device to use and an
-    optional torch.distributed process group over which the alignment classes are row-sharded."""
+             report_posterior: bool = False, device=None, group=None, bootstrap: int = 0, bootstrap_seed: int = 0) -> None:
+    """Quantify expected read counts.  Additions: `device` / `group`, the CUDA device to use and an optional
+    torch.distributed process group over which the alignment classes are row-sharded; `bootstrap` / `bootstrap_seed`,
+    replicates written after the reports (see `_write_bootstrap`; 0 = none)."""
     if group_file is None:
         group_file = os.path.join(DATA_DIR, "ref.gene2transcripts.tsv")
         if not os.path.exists(group_file):
@@ -176,4 +191,5 @@ def quantify(alignment_file: str, group_file: str = None, length_file: str = Non
                        report_posterior, notes_t=gtcall_t, notes_g=gtcall_g,
                        unmasked=None if masked_on_host else aln_mat,
                        unmasked_pattern=em_factory._pattern if reuse_pattern else None)
+        _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters)
     logger.debug("Done")

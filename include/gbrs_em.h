@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define GBRS_EM_ABI_VERSION 7
+#define GBRS_EM_ABI_VERSION 8
 #define GBRS_HPAD 8 /* haplotype slots per locus line */
 #define GBRS_KMAX 8 /* classes with up to this many (class, locus) pairs take the fixed-width row pass */
 #define GBRS_DEEP_LOCUS_ITEMS 8 /* a locus with more partial sums (column-pass items / tile slots) than this is summed by a
@@ -288,6 +288,13 @@ typedef struct {
   double* err_log;  /* [max_iters_cap] err_sum per iteration */
   double* scal;     /* [8] device scalars */
   int32_t* ctrl;    /* [16] control block, see GBRS_CTRL_* */
+  /* Row-pass variant (last, so that the kernels' parameter offsets of the fields above stay as they were).
+     1: a class of count 0 is absent -- the model-4 row pass gives it weight 0 without dividing, so a class whose entries
+     all have theta 0 contributes nothing instead of 0 / 0 (models 1-3 guard their divisions already).  This is the EM on
+     the matrix with the count-0 classes removed, as a bootstrap replicate needs it (gbrs_boot_resample).  A class with a
+     positive count and a zero normaliser still raises GBRS_E_NUMERIC.  0 (default): the ordinary row pass. */
+  int32_t zero_count_absent;
+  int32_t reserved;  /* 0 */
 } gbrs_em_dev;
 
 #define GBRS_PART_SLOTS 4096 /* [0, 2048): block partial sums of the isoform totals; [2048, 4096): of the error */
@@ -339,6 +346,29 @@ int gbrs_em_posterior_scratch_bytes(const gbrs_em_dev* d, int model, int64_t N, 
 int gbrs_em_posterior(const gbrs_em_dev* d, int model, const double* theta_src, const uint32_t* class_id, int64_t N,
                       const int64_t* const* indptr, const void* const* indices, int32_t index_bytes,
                       double* const* values, void* scratch, int64_t scratch_bytes, void* stream);
+/* ------------------------------------------------------------------------------------------------------------------
+ * Bootstrap replicates (DESIGN.md section 7.2): resample the M = sum(count) reads with replacement on the device and
+ * write the replicate's class counts, so that the EM can be rerun on them.  The reference has no counterpart.
+ * Replicate `replicate` of `seed` is fixed by (seed, replicate, count) alone:
+ *   draw pair j (j = 0 .. ceil(M/2)-1) = Philox4x32-10 with counter (j & 0xffffffff, j >> 32, replicate, 0) and key
+ *     (seed & 0xffffffff, seed >> 32) -> words x0..x3; draw 2j = x0 | x1 << 32, draw 2j+1 = x2 | x3 << 32 (unused if M is
+ *     odd and 2j+1 = M);
+ *   draw u is read k = floor(u * M / 2^64), which lands in the first input class n with prefix[n] > k;
+ *   the replicate's count of input class n is the number of draws landing in it (integers summing to M).
+ * `prefix` (device, int64 [N]) is the inclusive prefix sum of the input counts in input class order; 1 <= M =
+ * prefix[N-1] <= 2^53, N < 2^32.  gbrs_boot_guide builds, in `scratch`, a guide table (entry g: the class of read
+ * floor(g * M / G), G = the smallest power of two >= N, at most 2^24) so that each search starts within a few classes;
+ * it is built once per (prefix, N, M) and read by every gbrs_boot_resample call on that scratch.  gbrs_boot_resample
+ * then counts the draws of one replicate (integer atomics: exact and independent of order) and writes
+ * count_out[p] = count of input class class_id[p] for the packed classes p < n_classes (`class_id`: the packer's array of
+ * that name), ready to be the `count` of a descriptor.  `scratch` (device, 256-byte aligned) holds at least
+ * gbrs_boot_scratch_bytes(N) bytes.  Both calls are asynchronous on `stream`. */
+int gbrs_boot_scratch_bytes(int64_t N, int64_t* bytes);
+int gbrs_boot_guide(const int64_t* prefix, int64_t N, int64_t M, void* scratch, int64_t scratch_bytes, void* stream);
+int gbrs_boot_resample(const int64_t* prefix, int64_t N, int64_t M, uint64_t seed, uint32_t replicate,
+                       const uint32_t* class_id, int64_t n_classes, void* scratch, int64_t scratch_bytes, double* count_out,
+                       void* stream);
+
 /* Device-to-device copy of the current theta (previous = 0) or of the other half of the ping-pong (previous = 1: after
  * an update, the theta that entered it) into dst [T][8]; the parity is read on the device, nothing synchronises. */
 int gbrs_em_copy_theta(const gbrs_em_dev* d, int previous, double* dst, void* stream);
