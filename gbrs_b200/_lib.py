@@ -19,6 +19,9 @@ ABI_VERSION = 8
 CTRL_ITERS, CTRL_DONE, CTRL_ERROR, CTRL_PARITY, CTRL_MAX_ITERS, CTRL_PREPARED = range(6)
 SCAL_ERR, SCAL_SUM_PREV, SCAL_TARGET, SCAL_SUM_CUR = range(4)
 
+BOOT_TPM, BOOT_COUNTS, BOOT_SHARE = range(3)  # gbrs_boot_derive quantities
+BOOT_MAX_QUANTILES, BOOT_SUMMARY_MAX_B = 16, 16384
+
 GBRS_OK, GBRS_E_ARG, GBRS_E_LIMIT, GBRS_E_CUDA, GBRS_E_NUMERIC, GBRS_E_NOMEM, GBRS_E_STATE = 0, -1, -2, -3, -4, -5, -6
 
 
@@ -147,6 +150,10 @@ SYMBOLS = {
     "gbrs_boot_guide": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
     "gbrs_boot_resample": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_int64,
                                      C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "gbrs_boot_derive": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                   C.c_int32, C.c_void_p, C.c_void_p]),
+    "gbrs_boot_summarize": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     "gbrs_write_table": (C.c_int, [C.c_char_p, C.c_char_p, C.POINTER(C.c_char_p), C.c_int64, C.c_void_p, C.c_int32,
                                    C.POINTER(C.c_char_p), C.c_void_p, C.c_int32]),
     "gbrs_parse_lengths": (C.c_int, [C.c_char_p, C.POINTER(C.c_char_p), C.c_int64, C.POINTER(C.c_char_p), C.c_int32,

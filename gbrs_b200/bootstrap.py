@@ -108,3 +108,129 @@ class BootstrapResult:
         isoforms_expected_read_counts and, with groups, gname, genes_tpm, genes_expected_read_counts."""
         with open(path, "wb") as fh:  # np.savez would append ".npz" to a name without it
             np.savez(fh, **self.arrays())
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# summaries (EMfactory.bootstrap_summary, DESIGN.md section 7.3)
+# ---------------------------------------------------------------------------------------------------------------------
+SUMMARY_MAX_REPLICATES = 16384  # GBRS_BOOT_SUMMARY_MAX_B of gbrs_boot_summarize: a column is sorted in shared memory
+LEVELS = ("isoforms", "genes")
+QUANTITIES = ("tpm", "expected_read_counts", "allelic_share")
+
+
+def interval_quantiles(interval: float) -> np.ndarray:
+    """The quantiles of a central interval: (1 - interval) / 2, 0.5, 1 - (1 - interval) / 2."""
+    lo = (1.0 - float(interval)) / 2.0
+    return np.array([lo, 0.5, 1.0 - lo])
+
+
+def summarize_on_device(lib, stream, theta_all, acc_all, H: int, interval: float, genes=None) -> dict:
+    """gbrs_boot_derive + gbrs_boot_summarize for every (level, quantity), one at a time through one [B][E] buffer.
+    `theta_all` / `acc_all`: [B][T][8] device tensors; `genes`: (gene_ptr, gene_loci, number of real genes) or None;
+    `stream`: a stream of the tensors' device, on which the kernels run (that device is made current for the calls).
+    -> {(level, quantity): {"mean", "sd": [C, L], "q": [3, C, L], "n": int64 [L] (shares only)}} on the host, C = H + 1
+    (the last row is the total column) or H for shares."""
+    import ctypes as C
+
+    import torch
+
+    from . import _lib
+
+    B, T = int(theta_all.shape[0]), int(theta_all.shape[1])
+    q = interval_quantiles(interval)
+    dev = theta_all.device
+    # the launches go to the current device: make it the replicates' one (the factory's device need not be current)
+    with torch.cuda.device(dev):
+        values = torch.empty(B * T * (H + 1), dtype=torch.float64, device=dev)
+        out = {}
+        for level in LEVELS:
+            if level == "genes" and genes is None:
+                continue
+            gp, gl, L = (None, None, T) if level == "isoforms" else (C.c_void_p(genes[0].data_ptr()),
+                                                                    C.c_void_p(genes[1].data_ptr()), int(genes[2]))
+            for quantity, code in zip(QUANTITIES, (_lib.BOOT_TPM, _lib.BOOT_COUNTS, _lib.BOOT_SHARE)):
+                rows = H if code == _lib.BOOT_SHARE else H + 1
+                E = rows * L
+                src = acc_all if code == _lib.BOOT_COUNTS else theta_all
+                mean = torch.empty(E, dtype=torch.float64, device=dev)
+                sd = torch.empty(E, dtype=torch.float64, device=dev)
+                qo = torch.empty((len(q), E), dtype=torch.float64, device=dev)
+                n = torch.empty(E, dtype=torch.int32, device=dev)
+                _lib.check(lib.gbrs_boot_derive(C.c_void_p(src.data_ptr()), B, T, H, code, gp, gl, L if gp else 0,
+                                                C.c_void_p(values.data_ptr()), stream))
+                _lib.check(lib.gbrs_boot_summarize(C.c_void_p(values.data_ptr()), B, E, q.ctypes.data, len(q),
+                                                   C.c_void_p(mean.data_ptr()), C.c_void_p(sd.data_ptr()),
+                                                   C.c_void_p(qo.data_ptr()), C.c_void_p(n.data_ptr()), stream))
+                st = {"mean": mean.cpu().numpy().reshape(rows, L), "sd": sd.cpu().numpy().reshape(rows, L),
+                      "q": qo.cpu().numpy().reshape(len(q), rows, L)}
+                if code == _lib.BOOT_SHARE:  # whether a share is defined depends on the locus alone
+                    st["n"] = n.cpu().numpy().reshape(rows, L)[0].astype(np.int64)
+                out[(level, quantity)] = st
+    return out
+
+
+def _label(x: float) -> str:
+    return f"{x:.6g}"
+
+
+class BootstrapSummary:
+    """Statistics of B bootstrap replicates per element, over the replicates in the order given.
+      replicates, seed, model, total_reads, num_iters, interval, quantiles   as in BootstrapResult; quantiles =
+                                                                          interval_quantiles(interval)
+      stats[(level, quantity)]   level in LEVELS (genes only with groups), quantity in QUANTITIES:
+          "mean", "sd"  float64 [C, L]; "q" float64 [3, C, L] (quantiles in order); "n" int64 [L] for allelic_share
+          (replicates in which the locus' share is defined).  Rows: the haplotypes, then for tpm / expected_read_counts the
+          total column.
+      result   the BootstrapResult of the same replicates (keep_replicates=True), else None.
+    `write(outbase)` writes one table per (level, quantity)."""
+
+    def __init__(self, replicates, seed, model, total_reads, num_iters, interval, stats, lname=None, hname=None,
+                 gname=None, result=None):
+        self.replicates = np.asarray(replicates, dtype=np.int64)
+        self.seed, self.model, self.total_reads = int(seed), int(model), int(total_reads)
+        self.num_iters = np.asarray(num_iters, dtype=np.int64)
+        self.interval = float(interval)
+        self.quantiles = interval_quantiles(interval)
+        self.stats = stats
+        self.lname, self.hname, self.gname = lname, hname, gname
+        self.result = result
+
+    def __len__(self):
+        return int(self.replicates.shape[0])
+
+    def header(self, quantity: str, notes: bool = False) -> str:
+        cols = list(self.hname) + ([] if quantity == "allelic_share" else ["total"])
+        stats = ["mean", "sd"] + ["q" + _label(x) for x in self.quantiles]
+        head = ["locus"] + [f"{c}.{s}" for c in cols for s in stats]
+        if quantity == "allelic_share":
+            head.append("n")
+        if notes:
+            head.append("notes")
+        return "\t".join(head)
+
+    def columns(self, level: str, quantity: str) -> np.ndarray:
+        """[columns][loci] of the table: per haplotype (and total) mean, sd and the quantiles; n for shares."""
+        st = self.stats[(level, quantity)]
+        cols = []
+        for c in range(st["mean"].shape[0]):
+            cols += [st["mean"][c], st["sd"][c]] + [st["q"][j][c] for j in range(st["q"].shape[0])]
+        if "n" in st:
+            cols.append(st["n"].astype(np.float64))
+        return np.vstack(cols)
+
+    def write(self, outbase, notes_t=None, notes_g=None) -> list:
+        """{outbase}.bootstrap.{isoforms,genes}.{tpm,expected_read_counts,allelic_share}.summary, one row per locus in
+        input order, numbers formatted as the point reports format them.  Returns the paths written."""
+        from . import utils
+
+        paths = []
+        for level, names, notes in (("isoforms", self.lname, notes_t), ("genes", self.gname, notes_g)):
+            for quantity in QUANTITIES:
+                if (level, quantity) not in self.stats:
+                    continue
+                path = f"{outbase}.bootstrap.{level}.{quantity}.summary"
+                with open(path, "w") as fh:
+                    fh.write(self.header(quantity, notes is not None) + "\n")
+                    utils.write_table_rows(fh, names, self.columns(level, quantity), notes=notes)
+                paths.append(path)
+        return paths

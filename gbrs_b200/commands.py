@@ -40,6 +40,8 @@ def quantify(
     report_posterior: Annotated[bool, typer.Option("-w", "--report-posterior", help="whether to report posterior probabilities")] = False,
     bootstrap: Annotated[int, typer.Option("--bootstrap", help="bootstrap replicates, written to <outbase>.bootstrap.npz after the reports (default: 0 = none)")] = 0,
     bootstrap_seed: Annotated[int, typer.Option("--bootstrap-seed", help="seed of the bootstrap replicates (default: 0)")] = 0,
+    bootstrap_output: Annotated[str, typer.Option("--bootstrap-output", help="what --bootstrap writes: npz (the replicates), summary (mean / sd / interval tables) or both (default: npz)")] = "npz",
+    bootstrap_interval: Annotated[float, typer.Option("--bootstrap-interval", help="central interval of the bootstrap summary tables (default: 0.95)")] = 0.95,
     verbose: Annotated[int, typer.Option("-v", "--verbose", count=True, help="specify multiple times for more verbose output")] = 0,
 ) -> None:
     logger = utils.configure_logging("gbrs", verbose)
@@ -54,7 +56,8 @@ def quantify(
             genotype_file=str(genotype_file) if genotype_file else None,
             outbase=outbase, multiread_model=multiread_model, pseudocount=pseudocount, max_iters=max_iters,
             tolerance=tolerance, report_alignment_counts=report_alignment_counts, report_posterior=report_posterior,
-            bootstrap=bootstrap, bootstrap_seed=bootstrap_seed)
+            bootstrap=bootstrap, bootstrap_seed=bootstrap_seed, bootstrap_output=bootstrap_output,
+            bootstrap_interval=bootstrap_interval)
     except Exception as e:  # reference policy: log and return
         if logger.level == logging.DEBUG:
             logger.exception(e)
@@ -152,6 +155,8 @@ def run(
     report_posterior: Annotated[bool, typer.Option("-w", "--report-posterior", help="whether to report posterior probabilities")] = False,
     bootstrap: Annotated[int, typer.Option("--bootstrap", help="bootstrap replicates, written to <outbase>.bootstrap.npz after the reports (default: 0 = none)")] = 0,
     bootstrap_seed: Annotated[int, typer.Option("--bootstrap-seed", help="seed of the bootstrap replicates (default: 0)")] = 0,
+    bootstrap_output: Annotated[str, typer.Option("--bootstrap-output", help="what --bootstrap writes: npz (the replicates), summary (mean / sd / interval tables) or both (default: npz)")] = "npz",
+    bootstrap_interval: Annotated[float, typer.Option("--bootstrap-interval", help="central interval of the bootstrap summary tables (default: 0.95)")] = 0.95,
     verbose: Annotated[int, typer.Option("-v", "--verbose", count=True, help="specify multiple times for more verbose output")] = 0,
 ) -> None:
     """Flag surface of the reference's `emase run` (/root/reference/src/gbrs/emase/commands.py:315-356)."""
@@ -165,7 +170,8 @@ def run(
             length_file=str(length_file) if length_file else None, outbase=outbase, multiread_model=multiread_model,
             read_length=read_length, pseudocount=pseudocount, max_iters=max_iters, tolerance=tolerance,
             report_alignment_counts=report_alignment_counts, report_posterior=report_posterior,
-            bootstrap=bootstrap, bootstrap_seed=bootstrap_seed)
+            bootstrap=bootstrap, bootstrap_seed=bootstrap_seed, bootstrap_output=bootstrap_output,
+            bootstrap_interval=bootstrap_interval)
     except Exception as e:
         if logger.level == logging.DEBUG:
             logger.exception(e)

@@ -2603,6 +2603,186 @@ int check_boot(const int64_t* prefix, int64_t N, int64_t M, void* scratch, int64
   return GBRS_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Bootstrap summaries (gbrs_boot_derive / gbrs_boot_summarize; the contract is in include/gbrs_em.h and DESIGN.md 7.3).
+// Derive turns the replicates' [B][T][8] theta or numerator into the [B][E] values of one (level, quantity), element
+// e = h * L + l (h = H: the total column).  Summarize reduces each column of a [B][E] matrix: mean and sd in replicate
+// order, then a bitonic sort in shared memory (NaN last) for the quantiles, interpolated as numpy's method="linear".
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int kBootSumThreads = 512;               // k_bsum_tpm: one block per replicate row
+constexpr int kBootSummarySmem = 232448;           // dynamic shared memory of one summarize block (227 KB)
+constexpr int kBootSummaryMaxTile = 64;            // columns per summarize block
+
+__device__ __forceinline__ double boot_nan() { return __longlong_as_double(0x7FF8000000000000LL); }
+
+// one thread per (replicate, locus): the level's values x[h] (isoform: the locus line; gene: the sum over the gene's
+// loci in gene_loci order), then by `what`: 0 raw x[h] (TPM before scaling), 1 x[h] and the total column, 2 shares
+__global__ void __launch_bounds__(kThreads) k_bsum_level(const double* __restrict__ src, int64_t B, int32_t T, int32_t H,
+                                                         int32_t L, const uint32_t* __restrict__ gene_ptr,
+                                                         const uint32_t* __restrict__ gene_loci, int what,
+                                                         double* __restrict__ out) {
+  const int64_t total = B * L, stride = (int64_t) gridDim.x * blockDim.x;
+  const int64_t E = (int64_t) L * (what == 2 ? H : H + 1);
+  for (int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    const int64_t b = i / L, l = i - b * L;
+    const double* rep = src + (size_t) b * T * GBRS_HPAD;
+    double x[GBRS_HPAD];
+    if (!gene_ptr) {
+      load8(rep + (size_t) l * GBRS_HPAD, x);
+    } else {
+#pragma unroll
+      for (int h = 0; h < GBRS_HPAD; ++h) x[h] = 0.0;
+      for (uint32_t p = __ldg(gene_ptr + l), e = __ldg(gene_ptr + l + 1); p < e; ++p) {
+        double v[GBRS_HPAD];
+        load8(rep + (size_t) __ldg(gene_loci + p) * GBRS_HPAD, v);
+#pragma unroll
+        for (int h = 0; h < GBRS_HPAD; ++h) x[h] += v[h];
+      }
+    }
+    double* row = out + (size_t) b * E;
+    double sum = 0.0;
+#pragma unroll
+    for (int h = 0; h < GBRS_HPAD; ++h)
+      if (h < H) sum += x[h];
+#pragma unroll
+    for (int h = 0; h < GBRS_HPAD; ++h)
+      if (h < H) row[(int64_t) h * L + l] = what != 2 ? x[h] : (sum != 0.0 ? x[h] / sum : boot_nan());
+    if (what == 1) row[(int64_t) H * L + l] = sum;
+  }
+}
+
+// TPM: per replicate row (one block each), the sum S of its H * L raw values in a fixed order (thread-strided partial
+// sums, then a tree over the block), then value = x * (1e6 / S) and the total column
+__global__ void __launch_bounds__(kBootSumThreads) k_bsum_tpm(int64_t B, int32_t H, int32_t L, double* __restrict__ out) {
+  __shared__ double red[kBootSumThreads];
+  const int64_t n = (int64_t) H * L, E = (int64_t) (H + 1) * L;
+  for (int64_t b = blockIdx.x; b < B; b += gridDim.x) {
+    double* row = out + (size_t) b * E;
+    double s = 0.0;
+    for (int64_t i = threadIdx.x; i < n; i += blockDim.x) s += row[i];
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = kBootSumThreads / 2; w > 0; w >>= 1) {
+      if ((int) threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+      __syncthreads();
+    }
+    const double f = 1000000.0 / red[0];
+    for (int64_t l = threadIdx.x; l < L; l += blockDim.x) {
+      double t = 0.0;
+      for (int h = 0; h < H; ++h) {
+        const double v = __dmul_rn(row[(int64_t) h * L + l], f);
+        row[(int64_t) h * L + l] = v;
+        t += v;
+      }
+      row[(int64_t) H * L + l] = t;
+    }
+    __syncthreads();  // red[0] is rewritten by the next row
+  }
+}
+
+struct BootQuantiles {
+  double q[GBRS_BOOT_MAX_QUANTILES];
+};
+
+// compensated sum (Neumaier) in the order of the adds: the error of a column of 16k replicates stays at a few ulp
+struct BootSum {
+  double s = 0.0, c = 0.0;
+  __device__ __forceinline__ void add(double x) {
+    const double t = __dadd_rn(s, x);
+    c = __dadd_rn(c, fabs(s) >= fabs(x) ? __dadd_rn(__dadd_rn(s, -t), x) : __dadd_rn(__dadd_rn(x, -t), s));
+    s = t;
+  }
+  __device__ __forceinline__ double value() const { return __dadd_rn(s, c); }
+};
+
+// NaN sorts after every number
+__device__ __forceinline__ bool boot_after(double a, double b) { return a > b || (a != a && b == b); }
+
+// numpy.quantile(method="linear") of the n sorted numbers s[0..n): virtual index (n - 1) q, _lerp with its t >= 0.5
+// branch (numpy/lib/_function_base_impl.py), every operation rounded on its own (no FMA)
+__device__ __forceinline__ double boot_quantile(const double* s, int n, double q) {
+  const double v = __dmul_rn((double) (n - 1), q);
+  if (v >= (double) (n - 1)) return s[n - 1];
+  const double lo = floor(v);
+  const int i = (int) lo;
+  const double a = s[i], b = s[i + 1], t = __dadd_rn(v, -lo);
+  const double diff = __dadd_rn(b, -a);
+  return t >= 0.5 ? __dadd_rn(b, -__dmul_rn(diff, __dadd_rn(1.0, -t))) : __dadd_rn(a, __dmul_rn(diff, t));
+}
+
+// one block per tile of K columns (grid-stride over tiles): the tile is loaded transposed into shared memory (column k
+// at k * ld, ld = P + 1 with P the next power of two >= B, NaN padding), reads coalesced along E for each replicate;
+// thread k then takes mean, sd and n of column k in replicate order; a bitonic sort of all K columns follows, and the
+// quantiles are read off the sorted columns
+__global__ void __launch_bounds__(kThreads) k_boot_summarize(const double* __restrict__ values, int64_t B, int64_t E, int P,
+                                                             int K, const __grid_constant__ BootQuantiles Q, int nq, double* __restrict__ mean,
+                                                             double* __restrict__ sd, double* __restrict__ qout,
+                                                             int32_t* __restrict__ nout) {
+#ifdef GBRS_SIMT_EMULATION
+  static double s[kBootSummarySmem / sizeof(double)];
+#else
+  extern __shared__ double s[];
+#endif
+  const int ld = P + 1, half = P >> 1;
+  int half_bits = 0;
+  while ((1 << half_bits) < half) ++half_bits;
+  const int64_t n_tiles = (E + K - 1) / K;
+  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int64_t e0 = tile * K;
+    const int64_t cells = (int64_t) K * P;
+    for (int64_t i = threadIdx.x; i < cells; i += blockDim.x) {
+      const int64_t b = i / K;
+      const int k = (int) (i - b * K);
+      s[k * ld + b] = (b < B && e0 + k < E) ? values[(size_t) b * E + e0 + k] : boot_nan();
+    }
+    __syncthreads();
+    if ((int) threadIdx.x < K && e0 + threadIdx.x < E) {
+      const double* c = s + threadIdx.x * ld;
+      BootSum sum;
+      int n = 0;
+      for (int64_t b = 0; b < B; ++b)
+        if (c[b] == c[b]) { sum.add(c[b]); ++n; }
+      const double m = n > 0 ? sum.value() / n : boot_nan();
+      BootSum ss;
+      for (int64_t b = 0; b < B; ++b)
+        if (c[b] == c[b]) { const double dv = __dadd_rn(c[b], -m); ss.add(__dmul_rn(dv, dv)); }
+      const int64_t e = e0 + threadIdx.x;
+      mean[e] = m;
+      sd[e] = n > 1 ? sqrt(ss.value() / (n - 1)) : boot_nan();
+      if (nout) nout[e] = n;
+    }
+    __syncthreads();
+    for (int size = 2; size <= P; size <<= 1)
+      for (int st = size >> 1; st > 0; st >>= 1) {
+        for (int64_t i = threadIdx.x; i < (int64_t) K * half; i += blockDim.x) {
+          const int k = (int) (i >> half_bits), j = (int) (i & (half - 1));
+          const int lo = 2 * st * (j / st) + (j % st), hi = lo + st;
+          double* c = s + k * ld;
+          const double a = c[lo], b = c[hi];
+          if ((lo & size) == 0 ? boot_after(a, b) : boot_after(b, a)) { c[lo] = b; c[hi] = a; }
+        }
+        __syncthreads();
+      }
+    for (int64_t i = threadIdx.x; i < (int64_t) K * nq; i += blockDim.x) {
+      const int k = (int) (i % K), j = (int) (i / K);
+      const int64_t e = e0 + k;
+      if (e >= E) continue;
+      const double* c = s + k * ld;
+      int n = 0;  // the defined values are the sorted prefix
+      for (int step = P; step > 0; step >>= 1)
+        if (n + step <= P && c[n + step - 1] == c[n + step - 1]) n += step;
+      qout[(size_t) j * E + e] = n > 0 ? boot_quantile(c, n, Q.q[j]) : boot_nan();
+    }
+    __syncthreads();  // the next tile overwrites the columns
+  }
+}
+
+inline int boot_pow2(int64_t B) {
+  int P = 2;
+  while (P < B) P <<= 1;
+  return P;
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -3145,5 +3325,59 @@ extern "C" int gbrs_boot_resample(const int64_t* prefix, int64_t N, int64_t M, u
     k_boot_scatter<<<grid_for(n_classes), kThreads, 0, s>>>(hist, class_id, n_classes, count_out);
     GBRS_LAUNCH_CHECK("k_boot_scatter");
   }
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_boot_derive(const double* src, int64_t B, int32_t T, int32_t H, int32_t quantity, const uint32_t* gene_ptr,
+                                const uint32_t* gene_loci, int32_t n_genes, double* values, void* stream) {
+  if (!src || !values || B < 1 || T < 1 || H < 1 || H > GBRS_HPAD || quantity < GBRS_BOOT_TPM ||
+      quantity > GBRS_BOOT_SHARE || (gene_ptr != nullptr) != (gene_loci != nullptr) || (gene_ptr && n_genes < 1)) {
+    gbrs_set_error("gbrs_boot_derive: bad argument");
+    return GBRS_E_ARG;
+  }
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) { gbrs_set_error("gbrs_boot_derive: no CUDA device (there is no CPU fallback)"); return GBRS_E_CUDA; }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int32_t L = gene_ptr ? n_genes : T;
+  const int what = quantity == GBRS_BOOT_TPM ? 0 : quantity == GBRS_BOOT_COUNTS ? 1 : 2;
+  k_bsum_level<<<grid_for(B * L), kThreads, 0, s>>>(src, B, T, H, L, gene_ptr, gene_loci, what, values);
+  GBRS_LAUNCH_CHECK("k_bsum_level");
+  if (quantity == GBRS_BOOT_TPM) {
+    k_bsum_tpm<<<(int) (B < 65535 ? B : 65535), kBootSumThreads, 0, s>>>(B, H, L, values);
+    GBRS_LAUNCH_CHECK("k_bsum_tpm");
+  }
+  return GBRS_OK;
+}
+
+extern "C" int gbrs_boot_summarize(const double* values, int64_t B, int64_t E, const double* q, int32_t nq, double* mean,
+                                   double* sd, double* qout, int32_t* n, void* stream) {
+  if (!values || B < 1 || E < 0 || nq < 0 || nq > GBRS_BOOT_MAX_QUANTILES || (nq > 0 && (!q || !qout)) || !mean || !sd) {
+    gbrs_set_error("gbrs_boot_summarize: bad argument");
+    return GBRS_E_ARG;
+  }
+  if (B > GBRS_BOOT_SUMMARY_MAX_B) {
+    gbrs_set_error("gbrs_boot_summarize: at most " + std::to_string(GBRS_BOOT_SUMMARY_MAX_B) + " replicates");
+    return GBRS_E_LIMIT;
+  }
+  BootQuantiles Q{};
+  for (int j = 0; j < nq; ++j) {
+    if (!(q[j] >= 0.0 && q[j] <= 1.0)) { gbrs_set_error("gbrs_boot_summarize: quantiles must be in [0, 1]"); return GBRS_E_ARG; }
+    Q.q[j] = q[j];
+  }
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) { gbrs_set_error("gbrs_boot_summarize: no CUDA device (there is no CPU fallback)"); return GBRS_E_CUDA; }
+  if (E == 0) return GBRS_OK;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int P = boot_pow2(B);
+  const int64_t col_bytes = (int64_t) (P + 1) * (int64_t) sizeof(double);
+  int64_t K = kBootSummarySmem / col_bytes;
+  if (K > kBootSummaryMaxTile) K = kBootSummaryMaxTile;
+  if (K > E) K = E;
+  const int smem_bytes = (int) (K * col_bytes);
+  GBRS_CUDA(cudaFuncSetAttribute(k_boot_summarize, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+  const int64_t n_tiles = (E + K - 1) / K;
+  const int grid = (int) (n_tiles < (int64_t) sm_count() * 8 ? n_tiles : (int64_t) sm_count() * 8);
+  k_boot_summarize<<<grid, kThreads, smem_bytes, s>>>(values, B, E, P, (int) K, Q, nq, mean, sd, qout, n);
+  GBRS_LAUNCH_CHECK("k_boot_summarize");
   return GBRS_OK;
 }

@@ -1106,6 +1106,39 @@ class EMfactory:
         replicates run on their own device state: everything this factory reports afterwards is bit-identical to before.
         Refused (before any device work): row-sharded factories, weighted files, counts that are not non-negative
         integers or sum to more than 2^53, M = 0."""
+        reps, counts = self._check_bootstrap(replicates, model, seed, max_iters)
+        M, iters, theta_all, acc_all = self._replicate_loop(reps, counts, model, seed, pseudocount, tol, max_iters)
+        return self._host_result(reps, model, seed, M, iters, theta_all, acc_all)
+
+    def bootstrap_summary(self, replicates, model: int = 4, seed: int = 0, pseudocount: float = 0.0, tol: float = 0.0001,
+                          max_iters: int = 999, interval: float = 0.95,
+                          keep_replicates: bool = False) -> _boot.BootstrapSummary:
+        """Mean, standard deviation and percentile interval of the bootstrap replicates (DESIGN.md section 7.3), reduced on
+        the device: TPM, expected read counts and allelic shares at isoform and (with groups) gene level.  The replicates
+        are those of `bootstrap()` with the same arguments; `interval` in (0, 1) gives the quantiles (1 - interval) / 2,
+        0.5 and 1 - (1 - interval) / 2.  Nothing [B, H, T]-sized comes to the host unless `keep_replicates`, which also
+        returns `.result`, the BootstrapResult of `bootstrap()` bit for bit.  Refused as `bootstrap()` refuses, and for
+        fewer than 2 or more than `bootstrap.SUMMARY_MAX_REPLICATES` replicates or `interval` outside (0, 1)."""
+        reps, counts = self._check_bootstrap(replicates, model, seed, max_iters)
+        if not 0.0 < float(interval) < 1.0:
+            raise ValueError("the bootstrap interval must be in (0, 1)")
+        if not 2 <= reps.shape[0] <= _boot.SUMMARY_MAX_REPLICATES:
+            raise ValueError(f"bootstrap summaries need 2 to {_boot.SUMMARY_MAX_REPLICATES} replicates")
+        pat = self._pattern
+        p = self.probability
+        M, iters, theta_all, acc_all = self._replicate_loop(reps, counts, model, seed, pseudocount, tol, max_iters)
+        genes = None
+        if p.num_groups > 0:
+            genes = (pat.dev["gene_ptr"], pat.dev["gene_loci"], int(p.num_groups))
+        stats = _boot.summarize_on_device(pat.lib, pat.stream(), theta_all, acc_all, p.num_haplotypes, interval, genes)
+        result = None
+        if keep_replicates:
+            result = self._host_result(reps, model, seed, M, iters, theta_all, acc_all)
+        return _boot.BootstrapSummary(reps, int(seed), model, M, iters, float(interval), stats, lname=p.lname,
+                                      hname=p.hname, gname=p.gname if p.num_groups > 0 else None, result=result)
+
+    def _check_bootstrap(self, replicates, model, seed, max_iters):
+        """The refusals of bootstrap() (before any device work) -> (replicate indices, int64 input class counts)."""
         if model not in (1, 2, 3, 4):
             raise RuntimeError("The read normalization model should be 1, 2, 3, or 4.")
         if max_iters > ERR_LOG_CAP:
@@ -1118,16 +1151,21 @@ class EMfactory:
             raise NotImplementedError("bootstrap replicates of a weighted alignment file (stored values other than 1) "
                                       "are not supported")
         p = self.probability
-        T, H, N = p.shape
         if model != 4 and p.num_groups == 0:
             raise _lib.GbrsError("Group information matrix is missing.")
         reps = _boot.replicate_indices(replicates)
-        counts = _boot.read_counts_of(p.count, N)
-        M = int(counts.sum())
-        if M == 0:
+        counts = _boot.read_counts_of(p.count, p.shape[2])
+        if int(counts.sum()) == 0:
             raise ValueError("bootstrap needs at least one read (the counts sum to 0)")
         if not 0 <= int(seed) < 2 ** 64:
             raise ValueError("the bootstrap seed must fit 64 bits")
+        return reps, counts
+
+    def _replicate_loop(self, reps, counts, model, seed, pseudocount, tol, max_iters):
+        """The replicates of checked arguments on the replicate state -> (M, iteration counts, theta_all, acc_all), the
+        last two [B][T][8] device tensors."""
+        T, H, N = self.probability.shape
+        M = int(counts.sum())
         torch = _torch()
         pat = self._pattern
         pat.ensure_arrays(["class_id"])
@@ -1158,6 +1196,12 @@ class EMfactory:
                 iters[b] = n.value
                 _lib.check(lib.gbrs_em_copy_theta(C.byref(st.desc), 0, C.c_void_p(theta_all[b].data_ptr()), pat.stream()))
                 acc_all[b].copy_(st.acc)
+        return M, iters, theta_all, acc_all
+
+    def _host_result(self, reps, model, seed, M, iters, theta_all, acc_all) -> _boot.BootstrapResult:
+        p = self.probability
+        H = p.num_haplotypes
+        with _torch().cuda.device(self._pattern.device):
             theta = theta_all[:, :, :H].permute(0, 2, 1).contiguous().cpu().numpy()
             acc = acc_all[:, :, :H].permute(0, 2, 1).contiguous().cpu().numpy()
         return _boot.BootstrapResult(reps, int(seed), model, M, iters, theta, acc, grp_conv_mat=self.grp_conv_mat,

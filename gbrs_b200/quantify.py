@@ -10,6 +10,7 @@ import numpy as np
 
 from . import utils
 from .apm import AlignmentPropertyMatrix
+from .bootstrap import SUMMARY_MAX_REPLICATES
 from .emfactory import EMfactory
 
 DATA_DIR = os.getenv("GBRS_DATA", ".")
@@ -90,25 +91,51 @@ def _write_reports(em_factory, outbase, alignment_file, group_file, report_group
                                            pattern=unmasked_pattern)
 
 
-def _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters):
-    """`--bootstrap N`: N replicates (indices 0..N-1 of `bootstrap_seed`) after the point-estimate reports, written to
-    {outbase}.bootstrap.npz (BootstrapResult.save)."""
+BOOTSTRAP_OUTPUTS = ("npz", "summary", "both")
+
+
+def check_bootstrap_args(bootstrap, bootstrap_output, bootstrap_interval) -> None:
+    """The refusals of the bootstrap flags that need no data, checked before the input is loaded and the EM runs."""
+    if bootstrap_output not in BOOTSTRAP_OUTPUTS:
+        raise ValueError(f"--bootstrap-output must be one of {', '.join(BOOTSTRAP_OUTPUTS)}")
+    if not 0.0 < bootstrap_interval < 1.0:
+        raise ValueError("--bootstrap-interval must be in (0, 1)")
+    if bootstrap > 0 and bootstrap_output != "npz" and not 2 <= bootstrap <= SUMMARY_MAX_REPLICATES:
+        raise ValueError(f"bootstrap summaries need 2 to {SUMMARY_MAX_REPLICATES} replicates")
+
+
+def _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters,
+                     bootstrap_output="npz", bootstrap_interval=0.95, notes_t=None, notes_g=None):
+    """`--bootstrap N`: N replicates (indices 0..N-1 of `bootstrap_seed`) after the point-estimate reports.
+    `bootstrap_output`: "npz" writes them to {outbase}.bootstrap.npz (BootstrapResult.save); "summary" writes the
+    summary tables {outbase}.bootstrap.{isoforms,genes}.{tpm,expected_read_counts,allelic_share}.summary
+    (BootstrapSummary.write, interval `bootstrap_interval`); "both" writes both from one set of replicates."""
     if bootstrap <= 0:
         return
     path = f"{outbase}.bootstrap.npz"
-    logger.info(f"Running {bootstrap} bootstrap replicates (seed {bootstrap_seed}): {path}")
-    res = em_factory.bootstrap(bootstrap, model=multiread_model, seed=bootstrap_seed, pseudocount=pseudocount,
-                               tol=tolerance, max_iters=max_iters)
-    res.save(path)
+    kw = dict(model=multiread_model, seed=bootstrap_seed, pseudocount=pseudocount, tol=tolerance, max_iters=max_iters)
+    if bootstrap_output == "npz":
+        logger.info(f"Running {bootstrap} bootstrap replicates (seed {bootstrap_seed}): {path}")
+        em_factory.bootstrap(bootstrap, **kw).save(path)
+        return
+    logger.info(f"Running {bootstrap} bootstrap replicates (seed {bootstrap_seed}): {outbase}.bootstrap.*.summary")
+    summary = em_factory.bootstrap_summary(bootstrap, interval=bootstrap_interval,
+                                           keep_replicates=bootstrap_output == "both", **kw)
+    summary.write(outbase, notes_t=notes_t, notes_g=notes_g)
+    if bootstrap_output == "both":
+        summary.result.save(path)
 
 
 def run(alignment_file: str, group_file: str = None, length_file: str = None, outbase: str = "emase",
         multiread_model: int = 4, read_length: int = 100, pseudocount: float = 0.0, max_iters: int = 999,
         tolerance: float = 0.0001, report_alignment_counts: bool = False, report_posterior: bool = False,
-        device=None, group=None, bootstrap: int = 0, bootstrap_seed: int = 0) -> None:
+        device=None, group=None, bootstrap: int = 0, bootstrap_seed: int = 0, bootstrap_output: str = "npz",
+        bootstrap_interval: float = 0.95) -> None:
     """`emase run` workflow (reference `gbrs.emase.emase_utils.run`, emase/emase_utils.py:594-696): the same EM without
     the genotype restriction, with an explicit read length and no default group / length files.  `bootstrap` /
-    `bootstrap_seed`: replicates written after the reports (see `_write_bootstrap`; 0 = none)."""
+    `bootstrap_seed` / `bootstrap_output` / `bootstrap_interval`: replicates written after the reports (see
+    `_write_bootstrap`; 0 = none)."""
+    check_bootstrap_args(bootstrap, bootstrap_output, bootstrap_interval)
     report_group_counts = group_file is not None
     logger.info(f"Alignment File: {alignment_file}")
     logger.info(f"Group File: {group_file}")
@@ -126,17 +153,20 @@ def run(alignment_file: str, group_file: str = None, length_file: str = None, ou
         reuse_pattern = em_factory.world == 1 and em_factory._pattern.packed.has_genes
         _write_reports(em_factory, outbase, alignment_file, group_file, report_group_counts, report_alignment_counts,
                        report_posterior, unmasked=aln_mat, unmasked_pattern=em_factory._pattern if reuse_pattern else None)
-        _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters)
+        _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters,
+                         bootstrap_output, bootstrap_interval)
     logger.debug("Done")
 
 
 def quantify(alignment_file: str, group_file: str = None, length_file: str = None, genotype_file: str = None,
              outbase: str = "gbrs.quantified", multiread_model: int = 4, pseudocount: float = 0.0,
              max_iters: int = 999, tolerance: float = 0.0001, report_alignment_counts: bool = False,
-             report_posterior: bool = False, device=None, group=None, bootstrap: int = 0, bootstrap_seed: int = 0) -> None:
+             report_posterior: bool = False, device=None, group=None, bootstrap: int = 0, bootstrap_seed: int = 0,
+             bootstrap_output: str = "npz", bootstrap_interval: float = 0.95) -> None:
     """Quantify expected read counts.  Additions: `device` / `group`, the CUDA device to use and an optional
-    torch.distributed process group over which the alignment classes are row-sharded; `bootstrap` / `bootstrap_seed`,
-    replicates written after the reports (see `_write_bootstrap`; 0 = none)."""
+    torch.distributed process group over which the alignment classes are row-sharded; `bootstrap` / `bootstrap_seed` /
+    `bootstrap_output` / `bootstrap_interval`, replicates written after the reports (see `_write_bootstrap`; 0 = none)."""
+    check_bootstrap_args(bootstrap, bootstrap_output, bootstrap_interval)
     if group_file is None:
         group_file = os.path.join(DATA_DIR, "ref.gene2transcripts.tsv")
         if not os.path.exists(group_file):
@@ -191,5 +221,6 @@ def quantify(alignment_file: str, group_file: str = None, length_file: str = Non
                        report_posterior, notes_t=gtcall_t, notes_g=gtcall_g,
                        unmasked=None if masked_on_host else aln_mat,
                        unmasked_pattern=em_factory._pattern if reuse_pattern else None)
-        _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters)
+        _write_bootstrap(em_factory, outbase, bootstrap, bootstrap_seed, multiread_model, pseudocount, tolerance, max_iters,
+                         bootstrap_output, bootstrap_interval, notes_t=gtcall_t, notes_g=gtcall_g)
     logger.debug("Done")

@@ -369,6 +369,36 @@ int gbrs_boot_resample(const int64_t* prefix, int64_t N, int64_t M, uint64_t see
                        const uint32_t* class_id, int64_t n_classes, void* scratch, int64_t scratch_bytes, double* count_out,
                        void* stream);
 
+/* Bootstrap summaries (DESIGN.md section 7.3): the spread of B replicates, reduced on the device.
+ * gbrs_boot_derive writes the [B][E] values of one (level, quantity) from `src` ([B][T][8], device: per replicate the
+ * theta of the EM for GBRS_BOOT_TPM / GBRS_BOOT_SHARE, the numerator `acc` for GBRS_BOOT_COUNTS).  The level is the
+ * isoforms (gene_ptr = gene_loci = NULL, L = T) or the genes g < n_genes = L of the packer's gene-major CSR `gene_ptr` /
+ * `gene_loci` (loci of gene ids >= n_genes, the ungrouped ones, take no part).  With x[h][l] the level's value of
+ * replicate b (a gene: summed over its loci in gene_loci order), element e = h * L + l of row b is
+ *   GBRS_BOOT_COUNTS  x[h][l] for h < H, and at h = H the total sum_h x[h][l] (in h order)           E = (H + 1) L
+ *   GBRS_BOOT_TPM     x[h][l] * (1e6 / S), S the sum of the row's H * L values in a fixed tree order; total as above
+ *   GBRS_BOOT_SHARE   x[h][l] / sum_h' x[h'][l], NaN where that sum is 0                                E = H L
+ * Asynchronous on `stream`. */
+#define GBRS_BOOT_TPM 0
+#define GBRS_BOOT_COUNTS 1
+#define GBRS_BOOT_SHARE 2
+int gbrs_boot_derive(const double* src, int64_t B, int32_t T, int32_t H, int32_t quantity, const uint32_t* gene_ptr,
+                     const uint32_t* gene_loci, int32_t n_genes, double* values, void* stream);
+/* gbrs_boot_summarize reduces every column e of `values` ([B][E] doubles, device) over its n non-NaN entries:
+ *   mean[e] = sum / n, the sum compensated (Neumaier) and taken in row order;
+ *   sd[e] = sqrt(sum (x - mean)^2 / (n - 1)) (ddof 1, a second pass around that mean, its sum compensated the same way),
+ *     NaN if n < 2;
+ *   qout[j * E + e] = numpy.nanquantile(column, q[j], method="linear"), bit for bit (virtual index (n - 1) q, numpy's
+ *     _lerp with its t >= 0.5 branch, each operation rounded on its own);
+ *   n[e] = n (int32; `n` may be NULL).  Every statistic is NaN where n = 0.
+ * `q` is a host array of nq <= GBRS_BOOT_MAX_QUANTILES values in [0, 1]; the outputs are device arrays.  B <=
+ * GBRS_BOOT_SUMMARY_MAX_B (a column is sorted in shared memory), GBRS_E_LIMIT above.  Needs no scratch; asynchronous on
+ * `stream`; the same call gives the same bits. */
+#define GBRS_BOOT_MAX_QUANTILES 16
+#define GBRS_BOOT_SUMMARY_MAX_B 16384
+int gbrs_boot_summarize(const double* values, int64_t B, int64_t E, const double* q, int32_t nq, double* mean, double* sd,
+                        double* qout, int32_t* n, void* stream);
+
 /* Device-to-device copy of the current theta (previous = 0) or of the other half of the ping-pong (previous = 1: after
  * an update, the theta that entered it) into dst [T][8]; the parity is read on the device, nothing synchronises. */
 int gbrs_em_copy_theta(const gbrs_em_dev* d, int previous, double* dst, void* stream);
