@@ -841,92 +841,6 @@ int launch_m1_narrow(const gbrs_em_dev* d, cudaStream_t s) {
   return GBRS_OK;
 }
 
-// Model 1 for classes of 1..GBRS_KMAX pairs, eight lanes per class (opt-in: GBRS_M1_FIXED, not yet measured).  Lane h of a
-// group owns haplotype h: the theta line of a pair and the gene's per-haplotype totals are read as one 64-byte access
-// per group, the eight weights of a run are written as one 64-byte line, the class needs no row pointer (width bucket
-// addressing) and no data-dependent loop.  Every warp-level collective is executed unconditionally by all 32 lanes
-// (the four classes of a warp have different run structures): results are selected by predicate afterwards.
-template <int K>
-__device__ __forceinline__ void row_class_m1(const gbrs_em_dev& d, const double* __restrict__ th, int64_t n, bool valid,
-                                             int h, int lane) {
-  const uint32_t pair0 = (uint32_t) (d.bucket_pair0[K - 1] + (n - d.bucket_class0[K - 1]) * K);
-  const uint32_t* __restrict__ pw = d.pairs + pair0;
-  uint32_t w[K];
-#pragma unroll
-  for (int p = 0; p < K; ++p) w[p] = __ldg(pw + p);
-  const double c = __ldg(d.count + n);
-  int32_t g[K];
-  double gam[K], x[K];
-#pragma unroll
-  for (int p = 0; p < K; ++p) {
-    const uint32_t t = w[p] & kLocusMask;
-    g[p] = __ldg(d.gene_of + t);
-    gam[p] = d.gamma[t];
-    x[p] = ((w[p] >> (24 + h)) & 1u) ? th[(size_t) t * GBRS_HPAD + h] : 0.0;
-  }
-  // Dh of the run each pair belongs to, for this lane's haplotype (members added in pair order)
-  double Dh[K], hg[K], Hs[K];
-  bool any[K];
-#pragma unroll
-  for (int p = 0; p < K; ++p) {
-    double a = 0.0;
-#pragma unroll
-    for (int q = 0; q < K; ++q) a += (g[q] == g[p]) ? x[q] : 0.0;
-    Dh[p] = a;
-    const bool nz = a != 0.0;
-    const uint32_t bits = __ballot_sync(0xFFFFFFFFu, nz);
-    any[p] = ((bits >> (lane & 24)) & 0xFFu) != 0u;  // some haplotype of the run is alive
-    hg[p] = __ldg(d.gene_hap + (size_t) g[p] * GBRS_HPAD + h);
-    Hs[p] = group8_sum(nz ? hg[p] : 0.0);
-  }
-  double total = 0.0;
-#pragma unroll
-  for (int p = 0; p < K; ++p) {
-    const bool start = (p == 0) || (g[p] != g[p - 1]);
-    total += (start && any[p]) ? gam[p] : 0.0;
-  }
-  uint32_t run = __ldg(d.runptr + n);
-#pragma unroll
-  for (int p = 0; p < K; ++p) {
-    const bool start = (p == 0) || (g[p] != g[p - 1]);
-    if (start) {
-      if (p > 0) ++run;
-      if (valid) {
-        const double wg = (Hs[p] != 0.0) ? c * gam[p] / total / Hs[p] : 0.0;
-        d.weights[(size_t) run * GBRS_HPAD + h] = (Dh[p] != 0.0) ? wg * hg[p] / Dh[p] : 0.0;
-      }
-    }
-  }
-}
-
-// one launch per width K: narrow classes (the bulk) are not compiled for the register needs of the widest
-template <int K>
-__global__ void __launch_bounds__(kThreads) k_weights_m1_fixed(const __grid_constant__ gbrs_em_dev d) {
-  if (d.ctrl[GBRS_CTRL_DONE]) return;
-  const double* __restrict__ th = theta_cur(d);
-  const int lane = threadIdx.x & 31, h = lane & 7, grp = lane >> 3;
-  const int64_t warp = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int64_t n_warps = ((int64_t) gridDim.x * blockDim.x) >> 5;
-  const int64_t c0 = d.bucket_class0[K - 1], c1 = d.bucket_class0[K];
-  const int64_t units = (c1 - c0 + 3) >> 2;  // four classes per warp; the loop bounds are uniform over the warp
-  for (int64_t u = warp; u < units; u += n_warps) {
-    int64_t n = c0 + 4 * u + grp;
-    const bool valid = n < c1;
-    if (!valid) n = c1 - 1;  // idle group at the end of the bucket: recomputes the last class, stores nothing
-    row_class_m1<K>(d, th, n, valid, h, lane);
-  }
-}
-
-template <int K>
-int launch_m1_fixed(const gbrs_em_dev* d, cudaStream_t s) {
-  const int64_t n = d->bucket_class0[K] - d->bucket_class0[K - 1];
-  if (n > 0) {
-    k_weights_m1_fixed<K><<<resident_grid(k_weights_m1_fixed<K>, n * 8), kThreads, 0, s>>>(*d);
-    GBRS_LAUNCH_CHECK("k_weights_m1_fixed");
-  }
-  return GBRS_OK;
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
 // column pass: for every work item (<= item_len consecutive locus-major entries of ONE locus) the per-haplotype sum of
 // the weights of its entries.  8 lanes per item; lane j ends up holding haplotype j and writes wit[item][j].
@@ -2300,32 +2214,13 @@ int launch_row_pass(const gbrs_em_dev* d, int model, cudaStream_t s) {
       break;
     }
     default: {
-      // GBRS_M1_FIXED: eight lanes per class for the classes of up to GBRS_KMAX pairs (parity-tested, not yet timed)
-      static const bool m1_fixed = std::getenv("GBRS_M1_FIXED") != nullptr;
-      static const bool m1_generic = std::getenv("GBRS_M1_GENERIC") != nullptr;  // A/B knob: the round-1 row pass for all
-      if (!m1_fixed && !m1_generic) {
-        // default: narrow classes thread-per-class without row pointers, the rest through the generic CSR walk
-        const int64_t n_narrow = d->bucket_class0[kM1Narrow], n_rest = d->n_classes - n_narrow;
-        if (n_rest > 0) k_weights_m1<<<grid_for(n_rest), kThreads, 0, s>>>(*d, n_narrow);
-        int rcn = launch_m1_narrow<3>(d, s);
-        if (!rcn) rcn = launch_m1_narrow<2>(d, s);
-        if (!rcn) rcn = launch_m1_narrow<1>(d, s);
-        if (rcn) return rcn;
-        break;
-      }
-      const int64_t n_fixed = m1_fixed ? d->bucket_class0[GBRS_KMAX] : 0, n_long = d->n_classes - n_fixed;
-      if (n_fixed > 0) {  // widest first
-        int r8 = launch_m1_fixed<8>(d, s);
-        if (!r8) r8 = launch_m1_fixed<7>(d, s);
-        if (!r8) r8 = launch_m1_fixed<6>(d, s);
-        if (!r8) r8 = launch_m1_fixed<5>(d, s);
-        if (!r8) r8 = launch_m1_fixed<4>(d, s);
-        if (!r8) r8 = launch_m1_fixed<3>(d, s);
-        if (!r8) r8 = launch_m1_fixed<2>(d, s);
-        if (!r8) r8 = launch_m1_fixed<1>(d, s);
-        if (r8) return r8;
-      }
-      if (n_long > 0) k_weights_m1<<<grid_for(n_long), kThreads, 0, s>>>(*d, n_fixed);
+      // narrow classes thread-per-class without row pointers, the rest through the generic CSR walk
+      const int64_t n_narrow = d->bucket_class0[kM1Narrow], n_rest = d->n_classes - n_narrow;
+      if (n_rest > 0) k_weights_m1<<<grid_for(n_rest), kThreads, 0, s>>>(*d, n_narrow);
+      int rcn = launch_m1_narrow<3>(d, s);
+      if (!rcn) rcn = launch_m1_narrow<2>(d, s);
+      if (!rcn) rcn = launch_m1_narrow<1>(d, s);
+      if (rcn) return rcn;
       break;
     }
   }

@@ -11,7 +11,6 @@
 //
 //   transpose  the stored entries that survive the haplotype mask, re-laid locus-major (k_gp_col_len, scan, k_gp_gen), are
 //              stable-sorted by class id (cub::DeviceRadixSort, library); rowstart from the sorted keys (k_gp_rowstart).
-//              (First form, GBRS_PACK_TRANSPOSE=count: k_gp_count, scan, k_gp_scatter through per-class cursors.)
 //   merge      per class: OR the haplotype bits of equal loci (records arrive ordered) -> pair words, pair count, smallest loci
 //   order      classes of this shard by (min(pairs, 9) - 1, smallest locus, second-smallest locus), stable   cub::DeviceRadixSort (library)
 //   fill       rowptr / count / pairs in the new order, pairs sorted by (gene, locus), (class, gene) runs
@@ -66,21 +65,6 @@ struct Columns {            // the H CSC matrices on the device
   int64_t N;
 };
 
-// one warp per (haplotype, locus) column; f(class id, locus, haplotype) for every stored entry that survives the mask
-template <class F>
-__device__ __forceinline__ void for_each_entry(const Columns& c, F&& f) {
-  const int lane = threadIdx.x & 31;
-  const int64_t n_warps = ((int64_t) gridDim.x * blockDim.x) >> 5, n_cols = (int64_t) c.H * c.T;
-  for (int64_t col = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5; col < n_cols; col += n_warps) {
-    const int h = (int) (col / c.T), t = (int) (col - (int64_t) h * c.T);
-    if (c.hapmask && !((c.hapmask[t] >> h) & 1)) continue;
-    const int64_t* ip = c.indptr + (int64_t) h * (c.T + 1) + t;
-    const int64_t b = ip[0], e = ip[1];
-    const uint32_t* src = c.indices + c.hoff[h];
-    for (int64_t i = b + lane; i < e; i += 32) f(src[i], t, h);
-  }
-}
-
 __global__ void __launch_bounds__(kGpThreads) k_gp_narrow(const int64_t* __restrict__ in, uint32_t* __restrict__ out, int64_t n,
                                                          int64_t N, int* bad) {
   for (int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t) gridDim.x * blockDim.x) {
@@ -90,23 +74,7 @@ __global__ void __launch_bounds__(kGpThreads) k_gp_narrow(const int64_t* __restr
   }
 }
 
-__global__ void __launch_bounds__(kGpThreads) k_gp_count(const Columns c, uint32_t* __restrict__ nz, int* bad) {
-  for_each_entry(c, [&](uint32_t cls, int, int) {
-    if ((int64_t) cls >= c.N) *bad = 1;
-    else atomicAdd(nz + cls, 1u);
-  });
-}
-
-__global__ void __launch_bounds__(kGpThreads) k_gp_scatter(const Columns c, const uint32_t* __restrict__ rowstart,
-                                                          uint32_t* __restrict__ cursor, uint32_t* __restrict__ rec) {
-  for_each_entry(c, [&](uint32_t cls, int t, int h) {
-    if ((int64_t) cls >= c.N) return;
-    const uint32_t k = atomicAdd(cursor + cls, 1u);
-    rec[rowstart[cls] + k] = ((uint32_t) t << 3) | (uint32_t) h;
-  });
-}
-
-// ---- transposition by sorting (default): the stored entries, re-laid locus-major, are stable-sorted by class id -------
+// ---- transposition by sorting: the stored entries, re-laid locus-major, are stable-sorted by class id ----------------
 // column lengths in [locus][haplotype] order after the haplotype mask
 __global__ void __launch_bounds__(kGpThreads) k_gp_col_len(const Columns c, uint32_t* __restrict__ len) {
   const int64_t n_cols = (int64_t) c.H * c.T;
@@ -146,20 +114,8 @@ __global__ void __launch_bounds__(kGpThreads) k_gp_rowstart(const uint32_t* __re
   }
 }
 
-__device__ __forceinline__ void shell_sort(uint32_t* a, int n) {
-  for (int gap = n >> 1; gap > 0; gap = gap == 2 ? 1 : (int) (gap / 2.2)) {
-    for (int i = gap; i < n; ++i) {
-      const uint32_t v = a[i];
-      int j = i;
-      for (; j >= gap && a[j - gap] > v; j -= gap) a[j] = a[j - gap];
-      a[j] = v;
-    }
-  }
-}
-
-// per class: records (locus << 3 | hap) -> pair words (locus | mask << 24), compacted at the front of the class' segment
-// SORTED: the records of a class already come ordered by (locus, haplotype) (transposition by sorting)
-template <bool SORTED>
+// per class: records (locus << 3 | hap) -> pair words (locus | mask << 24), compacted at the front of the class' segment;
+// the records of a class come ordered by (locus, haplotype) from the transposition by sorting
 __global__ void __launch_bounds__(kGpThreads) k_gp_merge(int64_t N, const uint32_t* __restrict__ rowstart,
                                                         uint32_t* __restrict__ rec,
                                                         uint32_t* __restrict__ npair, uint32_t* __restrict__ minloc,
@@ -168,17 +124,6 @@ __global__ void __launch_bounds__(kGpThreads) k_gp_merge(int64_t N, const uint32
     const int n = (int) (rowstart[c + 1] - rowstart[c]);
     uint32_t* a = rec + rowstart[c];
     if (n == 0) { npair[c] = 0; minloc[c] = 0xFFFFFFFFu; secloc[c] = 0u; continue; }
-    if (SORTED) {
-    } else if (n <= 12) {  // insertion sort
-      for (int i = 1; i < n; ++i) {
-        const uint32_t v = a[i];
-        int j = i - 1;
-        for (; j >= 0 && a[j] > v; --j) a[j + 1] = a[j];
-        a[j + 1] = v;
-      }
-    } else {
-      shell_sort(a, n);
-    }
     int k = 0;
     for (int i = 0; i < n;) {
       const uint32_t t = a[i] >> 3;
@@ -523,14 +468,14 @@ int read_back(const T* dev, T* host, int64_t n, cudaStream_t s) {
 
 template <typename E>
 int build_entries(Arena& A, cudaStream_t s, int64_t n_pairs, int64_t n_entries, int64_t n_items, int64_t n_classes, int64_t n_runs,
-                  int64_t item_len, bool interleave, const unsigned long long* skey, const uint32_t* sval, const uint32_t* pairs,
+                  int64_t item_len, const unsigned long long* skey, const uint32_t* sval, const uint32_t* pairs,
                   const uint32_t* lptr, const uint32_t* lstart, const uint32_t* lpart, const uint32_t* ppart,
                   const uint32_t* runptr, const uint32_t* ric, const uint32_t* item_off, gbrs_device_pack* out) {
   constexpr int SH = 8 * (int) sizeof(E) - 8;
   (void) SH;
-  E* a = A.get<E>(n_entries, interleave ? "tmp:ent_cls" : "ent_cls");
-  E* b = A.get<E>(n_entries, interleave ? "tmp:ent_pair" : "ent_pair");
-  E* c = A.get<E>(n_entries, interleave ? "tmp:ent_run" : "ent_run");
+  E* a = A.get<E>(n_entries, "tmp:ent_cls");
+  E* b = A.get<E>(n_entries, "tmp:ent_pair");
+  E* c = A.get<E>(n_entries, "tmp:ent_run");
   if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
   if (n_entries > 0) {
     k_gp_fill_pad<E><<<gp_grid(n_entries), kGpThreads, 0, s>>>(n_entries, a, b, c, (E) n_classes, (E) n_pairs, (E) n_runs);
@@ -538,19 +483,16 @@ int build_entries(Arena& A, cudaStream_t s, int64_t n_pairs, int64_t n_entries, 
       k_gp_fill_entries<E><<<gp_grid(n_pairs), kGpThreads, 0, s>>>(n_pairs, skey, sval, pairs, lptr, lstart, lpart, ppart, runptr, ric, a,
                                                                  b, c);
   }
-  if (interleave) {
-    E* a1 = A.get<E>(n_entries, "ent_cls");
-    E* b1 = A.get<E>(n_entries, "ent_pair");
-    E* c1 = A.get<E>(n_entries, "ent_run");
-    if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
-    if (n_items > 0)
-      k_gp_interleave<E><<<gp_grid(n_items * 32), kGpThreads, 0, s>>>(n_items, item_len, item_off, a, b, c, a1, b1, c1);
-    a = a1; b = b1; c = c1;
-  }
+  E* a1 = A.get<E>(n_entries, "ent_cls");
+  E* b1 = A.get<E>(n_entries, "ent_pair");
+  E* c1 = A.get<E>(n_entries, "ent_run");
+  if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
+  if (n_items > 0)
+    k_gp_interleave<E><<<gp_grid(n_items * 32), kGpThreads, 0, s>>>(n_items, item_len, item_off, a, b, c, a1, b1, c1);
   GP_CUDA(cudaGetLastError());
-  out->ent_cls = a;
-  out->ent_pair = b;
-  out->ent_run = c;
+  out->ent_cls = a1;
+  out->ent_pair = b1;
+  out->ent_run = c1;
   return GBRS_OK;
 }
 
@@ -643,9 +585,7 @@ extern "C" int gbrs_pack_device(const gbrs_pack_input* in, gbrs_alloc_fn alloc, 
   if (d_count_in) GP_CUDA(cudaMemcpyAsync(d_count_in, in->count, sizeof(double) * (size_t) N, cudaMemcpyHostToDevice, s));
 
   // ---- transposition: CSC columns -> class rows --------------------------------------------------------------------------
-  uint32_t* nz = A.get<uint32_t>(N + 1, "tmp:nz");
   uint32_t* rowstart = A.get<uint32_t>(N + 1, "tmp:rowstart");
-  uint32_t* cursor = A.get<uint32_t>(N + 1, "tmp:cursor");
   uint32_t* npair = A.get<uint32_t>(N + 1, "tmp:npair");
   uint32_t* minloc = A.get<uint32_t>(N + 1, "tmp:minloc");
   uint32_t* secloc = A.get<uint32_t>(N + 1, "tmp:secloc");
@@ -653,46 +593,33 @@ extern "C" int gbrs_pack_device(const gbrs_pack_input* in, gbrs_alloc_fn alloc, 
   int64_t* d_lohi = A.get<int64_t>(2, "tmp:lohi");
   unsigned long long* d_stats = A.get<unsigned long long>(8, "tmp:stats");
   if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
-  GP_CUDA(cudaMemsetAsync(nz, 0, sizeof(uint32_t) * (size_t) (N + 1), s));
-  GP_CUDA(cudaMemsetAsync(cursor, 0, sizeof(uint32_t) * (size_t) (N + 1), s));
   GP_CUDA(cudaMemsetAsync(rowstart, 0, sizeof(uint32_t), s));
   GP_CUDA(cudaMemsetAsync(d_stats, 0, sizeof(unsigned long long) * 8, s));
   const int col_grid = gp_grid((int64_t) H * T * 32);
-  const char* tr_env = std::getenv("GBRS_PACK_TRANSPOSE");
-  if (tr_env && std::string(tr_env) == "count") {
-    // A/B knob: the first form -- count per class, scan, scatter through per-class cursors (63 M atomics with a returned
-    // value: 3.0 ms at C2), then every class sorts its records (1.4 ms)
-    k_gp_count<<<col_grid, kGpThreads, 0, s>>>(col, nz, d_bad);
-    if (N > 0)
-      if (int rc = inclusive_scan_into(A, nz, rowstart + 1, N, s)) return rc;
-    k_gp_scatter<<<col_grid, kGpThreads, 0, s>>>(col, rowstart, cursor, rec);
-    if (N > 0) k_gp_merge<false><<<gp_grid(N), kGpThreads, 0, s>>>(N, rowstart, rec, npair, minloc, secloc);
-  } else {
-    // by sorting: the entries that survive the mask, re-laid locus-major (column starts by a scan over the T x H column
-    // lengths), are stable-sorted by class id (library radix sort over the bits of N); the records of a class then arrive
-    // ordered by (locus, haplotype) and merging them is one linear pass -- no atomics, no per-class sorts
-    const int64_t n_cols = (int64_t) H * T;
-    int64_t n_kept = 0;
-    for (int t = 0; t < T; ++t)
-      for (int h = 0; h < H; ++h)
-        if (!in->locus_hapmask || ((in->locus_hapmask[t] >> h) & 1)) n_kept += in->indptr[h][t + 1] - in->indptr[h][t];
-    uint32_t* collen = A.get<uint32_t>(n_cols + 1, "tmp:collen");
-    uint32_t* colstart = A.get<uint32_t>(n_cols + 1, "tmp:colstart");
-    uint32_t* keys = A.get<uint32_t>(n_kept, "tmp:keys");
-    uint32_t* keys2 = A.get<uint32_t>(n_kept, "tmp:keys2");
-    uint32_t* vals = A.get<uint32_t>(n_kept, "tmp:vals");
-    if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
-    GP_CUDA(cudaMemsetAsync(colstart, 0, sizeof(uint32_t), s));
-    k_gp_col_len<<<gp_grid(n_cols), kGpThreads, 0, s>>>(col, collen);
-    if (int rc = inclusive_scan_into(A, collen, colstart + 1, n_cols, s)) return rc;
-    k_gp_gen<<<col_grid, kGpThreads, 0, s>>>(col, colstart, keys, vals, d_bad);
-    int bits = 1;
-    while ((int64_t(1) << bits) < N) ++bits;
-    if (n_kept > 0)
-      if (int rc = sort_pairs(A, keys, keys2, vals, rec, n_kept, bits, s)) return rc;
-    k_gp_rowstart<<<gp_grid(n_kept + 1), kGpThreads, 0, s>>>(keys2, n_kept, N, rowstart);
-    if (N > 0) k_gp_merge<true><<<gp_grid(N), kGpThreads, 0, s>>>(N, rowstart, rec, npair, minloc, secloc);
-  }
+  // the entries that survive the mask, re-laid locus-major (column starts by a scan over the T x H column lengths), are
+  // stable-sorted by class id (library radix sort over the bits of N); the records of a class then arrive ordered by
+  // (locus, haplotype) and merging them is one linear pass -- no atomics, no per-class sorts
+  const int64_t n_cols = (int64_t) H * T;
+  int64_t n_kept = 0;
+  for (int t = 0; t < T; ++t)
+    for (int h = 0; h < H; ++h)
+      if (!in->locus_hapmask || ((in->locus_hapmask[t] >> h) & 1)) n_kept += in->indptr[h][t + 1] - in->indptr[h][t];
+  uint32_t* collen = A.get<uint32_t>(n_cols + 1, "tmp:collen");
+  uint32_t* colstart = A.get<uint32_t>(n_cols + 1, "tmp:colstart");
+  uint32_t* keys = A.get<uint32_t>(n_kept, "tmp:keys");
+  uint32_t* keys2 = A.get<uint32_t>(n_kept, "tmp:keys2");
+  uint32_t* vals = A.get<uint32_t>(n_kept, "tmp:vals");
+  if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
+  GP_CUDA(cudaMemsetAsync(colstart, 0, sizeof(uint32_t), s));
+  k_gp_col_len<<<gp_grid(n_cols), kGpThreads, 0, s>>>(col, collen);
+  if (int rc = inclusive_scan_into(A, collen, colstart + 1, n_cols, s)) return rc;
+  k_gp_gen<<<col_grid, kGpThreads, 0, s>>>(col, colstart, keys, vals, d_bad);
+  int bits = 1;
+  while ((int64_t(1) << bits) < N) ++bits;
+  if (n_kept > 0)
+    if (int rc = sort_pairs(A, keys, keys2, vals, rec, n_kept, bits, s)) return rc;
+  k_gp_rowstart<<<gp_grid(n_kept + 1), kGpThreads, 0, s>>>(keys2, n_kept, N, rowstart);
+  if (N > 0) k_gp_merge<<<gp_grid(N), kGpThreads, 0, s>>>(N, rowstart, rec, npair, minloc, secloc);
   k_gp_shard<<<1, 32, 0, s>>>(rowstart, N, in->shard_count, in->shard_rank, d_lohi);
 
   // ---- class order ---------------------------------------------------------------------------------------------------
@@ -711,13 +638,9 @@ extern "C" int gbrs_pack_device(const gbrs_pack_input* in, gbrs_alloc_fn alloc, 
     uint32_t* val1 = A.get<uint32_t>(N + 1, "tmp:val1");
     uint32_t* okey_g = A.get<uint32_t>(N + 1, "tmp:okey_g");
     if (A.failed) { gbrs_set_error("gbrs_pack_device: allocation failed"); return GBRS_E_NOMEM; }
-    if (std::getenv("GBRS_NO_SECLOC") != nullptr) {  // A/B knob: the round-1 order (width, smallest locus, class id)
-      if (int rc = sort_pairs(A, okey, okey2, oval, order, N, 32, s)) return rc;
-    } else {
-      if (int rc = sort_pairs(A, secloc, sec_sorted, oval, val1, N, 24, s)) return rc;
-      k_gp_gather_u32<<<gp_grid(N), kGpThreads, 0, s>>>(N, val1, okey, okey_g);
-      if (int rc = sort_pairs(A, okey_g, okey2, val1, order, N, 32, s)) return rc;
-    }
+    if (int rc = sort_pairs(A, secloc, sec_sorted, oval, val1, N, 24, s)) return rc;
+    k_gp_gather_u32<<<gp_grid(N), kGpThreads, 0, s>>>(N, val1, okey, okey_g);
+    if (int rc = sort_pairs(A, okey_g, okey2, val1, order, N, 32, s)) return rc;
   }
   k_gp_buckets<<<1, 32, 0, s>>>(okey2, N, d_buckets);
   GP_CUDA(cudaGetLastError());
@@ -807,11 +730,10 @@ extern "C" int gbrs_pack_device(const gbrs_pack_input* in, gbrs_alloc_fn alloc, 
   GP_CUDA(cudaMemcpyAsync(item_off + n_items, &n_entries32, sizeof(uint32_t), cudaMemcpyHostToDevice, s));
   const bool force64 = std::getenv("GBRS_FORCE_ENTRY64") != nullptr;
   const int entry_bytes = (!force64 && std::max({n_classes, n_pairs, n_runs}) + 1 < (int64_t(1) << 24)) ? 4 : 8;
-  const bool interleave = std::getenv("GBRS_NO_INTERLEAVE") == nullptr;
   int rc_e = entry_bytes == 4
-                 ? build_entries<uint32_t>(A, s, n_pairs, n_entries, n_items, n_classes, n_runs, item_len, interleave, ekey2, eval2, pairs,
+                 ? build_entries<uint32_t>(A, s, n_pairs, n_entries, n_items, n_classes, n_runs, item_len, ekey2, eval2, pairs,
                                            lptr, lstart, lpart, ppart, runptr, ric, item_off, out)
-                 : build_entries<unsigned long long>(A, s, n_pairs, n_entries, n_items, n_classes, n_runs, item_len, interleave, ekey2,
+                 : build_entries<unsigned long long>(A, s, n_pairs, n_entries, n_items, n_classes, n_runs, item_len, ekey2,
                                                      eval2, pairs, lptr, lstart, lpart, ppart, runptr, ric, item_off, out);
   if (rc_e) return rc_e;
 

@@ -227,8 +227,6 @@ extern "C" int gbrs_pack_create(const gbrs_pack_input* in, gbrs_pack_t* out) {
       // classes in that order).  Classes sharing their two smallest loci end up next to each other: a warp of the row pass
       // reads fewer distinct table rows, and the entries of a locus gather runs of consecutive weights in the column pass.
       std::vector<int64_t> sec_start((size_t) T + 2, 0);
-      if (std::getenv("GBRS_NO_SECLOC") != nullptr)  // A/B knob: the round-1 order (width, smallest locus, class id)
-        for (int64_t c = lo; c < hi; ++c) secloc[c] = 0u;
       for (int64_t c = lo; c < hi; ++c)
         if (npair[c]) ++sec_start[(size_t) secloc[c] + 1];
       for (int t = 0; t <= T; ++t) sec_start[(size_t) t + 1] += sec_start[(size_t) t];
@@ -493,27 +491,25 @@ extern "C" int gbrs_pack_create(const gbrs_pack_input* in, gbrs_pack_t* out) {
     // (L1 wavefronts), not by bytes.  So the ascending sequence is dealt round-robin instead: word 4j + i of a block
     // holds its (i * nq + j)-th smallest entry (nq = quads in the block), which makes every gather round read LANES
     // *consecutive* entries -- neighbouring classes, mostly the same one or two lines.
-    if (std::getenv("GBRS_NO_INTERLEAVE") == nullptr) {  // (knob for A/B measurements of this layout)
-      const int64_t nit = n_items;
+    const int64_t nit = n_items;
 #pragma omp parallel
-      {
-        std::vector<uint64_t> buf(128);
+    {
+      std::vector<uint64_t> buf(128);
 #pragma omp for schedule(dynamic, 256)
-        for (int64_t it = 0; it < nit; ++it) {
-          const int64_t b = P->item_off[it], e = P->item_off[it + 1];
-          const int64_t B = (e - b > item_len) ? 128 : 32;  // long items: a warp; short items: an 8-lane group
-          for (int64_t k = b; k < e; k += B) {
-            const int64_t m = std::min<int64_t>(B, e - k), nq = m / 4;
-            for (bigvec<uint8_t>* arr : {&P->ent_cls, &P->ent_pair, &P->ent_run}) {
-              if (entry_bytes == 4) {
-                uint32_t* w = reinterpret_cast<uint32_t*>(arr->data()) + k;
-                for (int64_t r = 0; r < m; ++r) buf[r] = w[r];
-                for (int64_t r = 0; r < m; ++r) w[4 * (r % nq) + r / nq] = (uint32_t) buf[r];
-              } else {
-                uint64_t* w = reinterpret_cast<uint64_t*>(arr->data()) + k;
-                for (int64_t r = 0; r < m; ++r) buf[r] = w[r];
-                for (int64_t r = 0; r < m; ++r) w[4 * (r % nq) + r / nq] = buf[r];
-              }
+      for (int64_t it = 0; it < nit; ++it) {
+        const int64_t b = P->item_off[it], e = P->item_off[it + 1];
+        const int64_t B = (e - b > item_len) ? 128 : 32;  // long items: a warp; short items: an 8-lane group
+        for (int64_t k = b; k < e; k += B) {
+          const int64_t m = std::min<int64_t>(B, e - k), nq = m / 4;
+          for (bigvec<uint8_t>* arr : {&P->ent_cls, &P->ent_pair, &P->ent_run}) {
+            if (entry_bytes == 4) {
+              uint32_t* w = reinterpret_cast<uint32_t*>(arr->data()) + k;
+              for (int64_t r = 0; r < m; ++r) buf[r] = w[r];
+              for (int64_t r = 0; r < m; ++r) w[4 * (r % nq) + r / nq] = (uint32_t) buf[r];
+            } else {
+              uint64_t* w = reinterpret_cast<uint64_t*>(arr->data()) + k;
+              for (int64_t r = 0; r < m; ++r) buf[r] = w[r];
+              for (int64_t r = 0; r < m; ++r) w[4 * (r % nq) + r / nq] = buf[r];
             }
           }
         }

@@ -96,9 +96,9 @@ def test_models_1_to_3_replicates_match_xref(H, model):
 
 
 def replicate_path(path):
-    """one replicate of model 4 (model 1 for the eight-lane row pass) on the 8-haplotype layout through `path`"""
+    """one replicate of model 4 on the 8-haplotype layout through `path`"""
     d = layouts.make_layout(8, 16)
-    kw, pc, gtmask, model = {}, 0.0, None, 4
+    kw, pc, gtmask = {}, 0.0, None
     if path == "pseudocount":
         pc = 0.5
     elif path == "genotype":
@@ -109,13 +109,11 @@ def replicate_path(path):
         kw = dict(locus_hapmask=hapmask_bytes(gtmask))
     elif path == "host-packer":
         kw = dict(pack="host")
-    elif path == "m1-fixed":
-        model = 1
     em = factory(d, pseudocount=pc, **kw)
     assert em._pattern.info["entry_bytes"] == (8 if path == "entry64" else 4)
     assert em._pattern.on_device == (path != "host-packer")
-    res = em.bootstrap([2], model=model, seed=9, pseudocount=pc, tol=TOL, max_iters=MAXIT)
-    check_replicates(d, res, model, pseudocount=pc, gtmask=gtmask, what=path)
+    res = em.bootstrap([2], model=4, seed=9, pseudocount=pc, tol=TOL, max_iters=MAXIT)
+    check_replicates(d, res, 4, pseudocount=pc, gtmask=gtmask, what=path)
 
 
 @pytest.mark.parametrize("path", ["pseudocount", "genotype", "host-packer", "entry64"])
@@ -123,28 +121,6 @@ def test_replicate_paths_match_xref(path, monkeypatch):
     if path == "entry64":
         monkeypatch.setenv("GBRS_FORCE_ENTRY64", "1")
     replicate_path(path)
-
-
-M1_FIXED_WORKER = r'''
-import os, sys
-sys.path.insert(0, os.environ["GBRS_ROOT"])
-from tests.test_bootstrap_gpu import replicate_path
-replicate_path("m1-fixed")
-print("M1-FIXED-OK")
-'''
-
-
-def test_replicate_model1_eight_lane_row_pass(tmp_path):
-    """GBRS_M1_FIXED (read once per process, so in a process of its own)."""
-    import subprocess
-    import sys
-
-    script = tmp_path / "worker.py"
-    script.write_text(M1_FIXED_WORKER)
-    env = dict(os.environ, GBRS_ROOT=os.path.dirname(os.path.dirname(os.path.abspath(__file__))), GBRS_M1_FIXED="1")
-    res = subprocess.run([sys.executable, str(script)], env=env, capture_output=True, text=True, timeout=900)
-    print("\n".join(line for line in res.stdout.splitlines() if "ELEMENTWISE" in line))
-    assert res.returncode == 0 and "M1-FIXED-OK" in res.stdout, res.stdout[-2000:] + res.stderr[-3000:]
 
 
 def test_replicates_do_not_depend_on_the_call_packer_or_layout():

@@ -1,12 +1,8 @@
 """Every output element of the device EM against the extended-precision reference (tests/xref.py), on layouts built to
 reach every kernel path (tests/layouts.py): each haplotype count H = 1..8, models 1-4, each code path of the update
-(two-pass kernels, 64-bit entry words, the fused tile kernel with wide and tiny tiles, row shards, the eight-lane model-1
-row pass).  The tolerance of an element is the error bound of tests/xref.py computed from the shape; zeros must match
+(two-pass kernels, 64-bit entry words, the fused tile kernel with wide and tiny tiles, row shards).  The tolerance of an element is the error bound of tests/xref.py computed from the shape; zeros must match
 exactly.  Each check prints one ELEMENTWISE line (largest relative error, and the bound at that shape) under `pytest -s`."""
 import ctypes as C
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -140,34 +136,3 @@ def test_gpu_run_to_convergence_elementwise(H):
     where = layouts.locus_kinds(em._pattern.packed)
     check(em.allelic_expression, want["theta"], rtol, f"H={H} run model {model} ({want['iters']} updates) theta", where)
     check(em.expected_read_counts(), want["counts"], rtol, f"H={H} run model {model} counts", where)
-
-
-M1_FIXED_WORKER = r'''
-import os, sys
-sys.path.insert(0, os.environ["GBRS_ROOT"])
-from tests.test_em_elementwise_gpu import check, factory, problem
-from tests import layouts
-from tests import xref as xr
-for H in range(1, 9):
-    d, gene_of, x, eff = problem(H)
-    em = factory(d, item_len=16)
-    layouts.assert_layout_covers(em._pattern.packed)
-    theta = xr.random_theta(x, seed=20 + H)
-    em.allelic_expression = theta
-    em.update_allelic_expression(model=1)
-    counts, theta1 = x.update(theta, 1, eff)
-    check(em.expected_read_counts(), counts, x.rtol_update(1), f"H={H} GBRS_M1_FIXED model 1 counts")
-    check(em.allelic_expression, theta1, x.rtol_update(1), f"H={H} GBRS_M1_FIXED model 1 theta")
-print("M1-FIXED-OK")
-'''
-
-
-def test_gpu_model1_eight_lane_row_pass_elementwise(tmp_path):
-    """GBRS_M1_FIXED (read once per process, so in a process of its own): one model-1 update at every H."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = tmp_path / "worker.py"
-    script.write_text(M1_FIXED_WORKER)
-    env = dict(os.environ, GBRS_ROOT=root, GBRS_M1_FIXED="1")
-    res = subprocess.run([sys.executable, str(script)], env=env, capture_output=True, text=True, timeout=900)
-    print(res.stdout)
-    assert res.returncode == 0 and "M1-FIXED-OK" in res.stdout, res.stdout[-2000:] + res.stderr[-3000:]

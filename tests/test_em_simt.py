@@ -457,15 +457,15 @@ print("TSAN-RUN-OK")
     assert "ThreadSanitizer: data race" not in res.stderr, res.stderr[-4000:]
 
 
-@pytest.mark.parametrize("knob", ["GBRS_FORCE_ENTRY64", "GBRS_NO_INTERLEAVE"])
+@pytest.mark.parametrize("knob", ["GBRS_FORCE_ENTRY64"])
 def test_emulated_alternative_layouts(knob, monkeypatch):
-    """64-bit locus-major entry words (what shards beyond 2^24 classes use) and the plain ascending entry order inside
-    work items: one update of every model on the forced layout against the oracle."""
+    """64-bit locus-major entry words (what shards beyond 2^24 classes use): one update of every model on the forced
+    layout against the oracle."""
     monkeypatch.setenv(knob, "1")
     d = synth.generate(T=90, N=1000, H=8, sample_index=13, wide_frac=0.04)
     gene_of = eo.gene_index(d.T, d.groups())
     pat = simt_em.HostPattern(synth.to_apm(d), gene_of=gene_of, item_len=8)
-    assert pat.info["entry_bytes"] == (8 if knob == "GBRS_FORCE_ENTRY64" else 4)
+    assert pat.info["entry_bytes"] == 8
     eff = eo.effective_length_table(d.lengths)
     theta = pat.prepare(eff)
     oapm = eo.apm_from_pairs(d.T, d.H, d.N, d.pair_class, d.pair_locus, d.pair_mask, d.count)
@@ -551,33 +551,3 @@ def test_emulated_library_on_random_shapes(seed):
         aln, uniq, lu = pats[0].alignment_counts()
         want = eo.alignment_counts(oapm)
         assert np.array_equal(aln, want["aln"]) and np.array_equal(uniq, want["uniq"]) and np.array_equal(lu, want["locus_uniq"])
-
-
-def test_emulated_model1_eight_lane_row_pass(monkeypatch):
-    """The opt-in model-1 row pass for classes of up to 8 pairs (GBRS_M1_FIXED: eight lanes per class, unconditional
-    warp collectives) on a private library instance: a reference golden, and a problem with wide classes (where the
-    generic kernel still serves the long classes) against the oracle and against the generic kernel."""
-    monkeypatch.delenv("GBRS_M1_FIXED", raising=False)
-    d = synth.generate(T=120, N=1500, H=8, sample_index=9, wide_frac=0.08)
-    gene_of = eo.gene_index(d.T, d.groups())
-    eff = eo.effective_length_table(d.lengths)
-    generic = simt_em.HostPattern(synth.to_apm(d), gene_of=gene_of, item_len=8, lib=simt_em.load_instance("m1generic"))
-    generic.prepare(eff)
-    og = generic.run(1, 0.0, 2)  # the launcher reads the knob once per library instance: this one stays generic
-    monkeypatch.setenv("GBRS_M1_FIXED", "1")
-    lib = simt_em.load_instance("m1fixed")
-    fixed = simt_em.HostPattern(synth.to_apm(d), gene_of=gene_of, item_len=8, lib=lib)
-    assert fixed.info["max_pairs_per_class"] > 8 > 0 < fixed.info["bucket_class0"][8]
-    fixed.prepare(eff)
-    of = fixed.run(1, 0.0, 2)
-    assert hp.relerr(of["counts"], og["counts"]) < 1e-13 and hp.relerr(of["theta"], og["theta"]) < 1e-13
-    assert np.abs(fixed.weights - generic.weights).max() > 0.0  # really another kernel (other summation order)
-    oapm = eo.apm_from_pairs(d.T, d.H, d.N, d.pair_class, d.pair_locus, d.pair_mask, d.count)
-    want = eo.run(oapm, eo.prepare(oapm, eff, 0.0), 1, eff, gene_of, tol=0.0, max_iters=2)
-    assert hp.relerr(of["counts"], want["counts"]) < 1e-12
-    g = hp.load_golden("em_small_m1_diploid")
-    dd = hp.synth_from_golden(g)
-    pat = pattern_for(g, dd, lib=lib)
-    pat.prepare(eo.effective_length_table(dd.lengths), g["pseudocount"])
-    out = pat.run(1, g["tol"], g["max_iters"])
-    assert out["iters"] == g["iters"] and hp.relerr(out["counts"], g["counts"]) < 1e-12

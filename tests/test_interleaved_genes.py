@@ -1,8 +1,8 @@
 """Genes whose loci interleave in locus order (tests/interleaved.py), on the CPU: the packed rows, runs and entries of the
 host packer and of the device packer (run through the host SIMT shim) against the input, and the gene-aware kernels of
 the EM library (tests/simt_em.py) element by element against the extended-precision reference of tests/xref.py: one
-update and a stand-alone E-step of models 1-3 (model 4 as a control), the eight-lane model-1 row pass, row shards, run()
-to convergence, a relabelling of the loci, the posterior, the gene-level alignment counts and a bootstrap replicate.
+update and a stand-alone E-step of models 1-3 (model 4 as a control), row shards, run() to convergence, a relabelling of
+the loci, the posterior, the gene-level alignment counts and a bootstrap replicate.
 
 Every test calls tests/layouts.assert_layout_covers and tests/interleaved.assert_genes_interleave on the pattern it
 runs, so the interleaving reaches every fixed-width row pass and both row-pointer widths."""
@@ -68,12 +68,10 @@ def test_host_packer_sorts_rows_by_gene_and_cuts_runs(H):
 
 
 @pytest.mark.parametrize("entry64", [False, True], ids=["entry32", "entry64"])
-@pytest.mark.parametrize("transpose", ["sort", "count"])
 @pytest.mark.parametrize("H", [2, 8])
-def test_emulated_device_packer_sorts_rows_by_gene_and_cuts_runs(H, transpose, entry64, monkeypatch):
-    """gpu_pack.cu through the host shim, both forms of its transposition: the structure against the input, and every
-    array bit-identical to the host packer's, at 32- and 64-bit entry words."""
-    monkeypatch.setenv("GBRS_PACK_TRANSPOSE", transpose)
+def test_emulated_device_packer_sorts_rows_by_gene_and_cuts_runs(H, entry64, monkeypatch):
+    """gpu_pack.cu through the host shim: the structure against the input, and every array bit-identical to the host
+    packer's, at 32- and 64-bit entry words."""
     if entry64:
         monkeypatch.setenv("GBRS_FORCE_ENTRY64", "1")
     d, gene_of, _, _ = problem(H)
@@ -141,24 +139,6 @@ def test_emulated_one_update_elementwise_entry64(H, monkeypatch):
     covers(d, pat.packed)
     pat.prepare(eff)
     one_update_each_model(pat, d, x, eff, xr.random_theta(x, seed=30 + H), f"H={H} entry64", None, estep=False)
-
-
-def test_emulated_model1_eight_lane_row_pass(monkeypatch):
-    """GBRS_M1_FIXED is read once per library instance: a private instance with the knob set, one model-1 update"""
-    monkeypatch.setenv("GBRS_M1_FIXED", "1")
-    lib = simt_em.load_instance("interleaved_m1fixed")
-    for H in (2, 8):
-        d, gene_of, x, eff = problem(H)
-        pat = simt_em.HostPattern(synth.to_apm(d), gene_of=gene_of, item_len=ITEM_LEN, lib=lib)
-        covers(d, pat.packed)
-        pat.prepare(eff)
-        theta = xr.random_theta(x, seed=20 + H)
-        tb = T8(theta, d.T)
-        pat.check(pat.lib.gbrs_em_set_theta(C.byref(pat.desc), tb.ctypes.data, None))
-        out = pat.run(1, tol=0.0, max_iters=1)
-        counts, theta1 = x.update(theta, 1, eff)
-        xr.assert_elementwise(out["counts"], counts, x.rtol_update(1), f"H={H} GBRS_M1_FIXED counts")
-        xr.assert_elementwise(out["theta"], theta1, x.rtol_update(1), f"H={H} GBRS_M1_FIXED theta")
 
 
 @pytest.mark.parametrize("R", [2, 3])

@@ -1,14 +1,11 @@
 """Genes whose loci interleave in locus order (tests/interleaved.py) on the device: the device packer's rows, runs and
 entries against the input and bit for bit against the host packer; every output element of the gene-aware EM paths
 against the extended-precision reference of tests/xref.py (one update and a stand-alone E-step of models 1-3 with model 4
-as a control, two-pass kernels and 64-bit entry words, the eight-lane model-1 row pass, row shards, run() to convergence,
+as a control, two-pass kernels and 64-bit entry words, row shards, run() to convergence,
 a relabelling of the loci); the posterior, the gene-level alignment counts, bootstrap replicates, and `quantify` end to
 end with the group file written out, with and without a genotype file.  Each check prints one ELEMENTWISE line under
 `pytest -s`."""
 import ctypes as C
-import os
-import subprocess
-import sys
 import time
 
 import numpy as np
@@ -121,36 +118,6 @@ def test_gpu_one_update_elementwise(H, path, monkeypatch):
         check(em.expected_read_counts(), counts, rtol, f"interleaved H={H} {path} model {model} counts")
         check(em.allelic_expression, theta1, rtol, f"interleaved H={H} {path} model {model} theta")
         assert not em.allelic_expression[:, d.zero_locus].any()
-
-
-M1_FIXED_WORKER = r'''
-import os, sys
-sys.path.insert(0, os.environ["GBRS_ROOT"])
-from tests.test_interleaved_genes_gpu import check, covers, factory, problem
-from tests import xref as xr
-for H in range(1, 9):
-    d, gene_of, x, eff = problem(H)
-    em = factory(d)
-    covers(d, em._pattern.packed)
-    theta = xr.random_theta(x, seed=20 + H)
-    em.allelic_expression = theta
-    em.update_allelic_expression(model=1)
-    counts, theta1 = x.update(theta, 1, eff)
-    check(em.expected_read_counts(), counts, x.rtol_update(1), f"interleaved H={H} GBRS_M1_FIXED model 1 counts")
-    check(em.allelic_expression, theta1, x.rtol_update(1), f"interleaved H={H} GBRS_M1_FIXED model 1 theta")
-print("M1-FIXED-OK")
-'''
-
-
-def test_gpu_model1_eight_lane_row_pass_elementwise(tmp_path):
-    """GBRS_M1_FIXED (read once per process, so in a process of its own): one model-1 update at every H"""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = tmp_path / "worker.py"
-    script.write_text(M1_FIXED_WORKER)
-    env = dict(os.environ, GBRS_ROOT=root, GBRS_M1_FIXED="1")
-    res = subprocess.run([sys.executable, str(script)], env=env, capture_output=True, text=True, timeout=900)
-    print(res.stdout)
-    assert res.returncode == 0 and "M1-FIXED-OK" in res.stdout, res.stdout[-2000:] + res.stderr[-3000:]
 
 
 @pytest.mark.parametrize("H", range(1, 9))

@@ -327,18 +327,16 @@ def test_emulated_device_packer_equals_host_packer(case):
 
 
 @pytest.mark.skipif(__import__("shutil").which("g++") is None, reason="g++ is needed to build the SIMT emulation")
-@pytest.mark.parametrize("transpose", ["sort", "count"])
-def test_emulated_device_packer_empty_classes_and_masked_loci(transpose, monkeypatch):
-    """Both forms of the device packer's transposition (stable sort of the locus-major entries / counting with per-class
-    cursors) on the corner cases of the class boundaries: classes without any alignment at the start, in the middle and at
-    the end of the id range, loci the genotype byte removes completely, and a matrix that is empty after masking."""
+def test_emulated_device_packer_empty_classes_and_masked_loci():
+    """The device packer's transposition (stable sort of the locus-major entries) on the corner cases of the class
+    boundaries: classes without any alignment at the start, in the middle and at the end of the id range, loci the
+    genotype byte removes completely, and a matrix that is empty after masking."""
     from scipy.sparse import csc_matrix
 
     from gbrs_b200 import AlignmentPropertyMatrix as APM
     from gbrs_b200.emfactory import PackedPattern
     from tests import simt_em
 
-    monkeypatch.setenv("GBRS_PACK_TRANSPOSE", transpose)
     rng = np.random.default_rng(5)
     T, H, N = 23, 4, 400
     dense = (rng.random((H, N, T)) < 0.04).astype(np.float64)

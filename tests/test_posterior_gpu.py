@@ -1,7 +1,7 @@
 """EMfactory.posterior_probability() on the device, element by element against the extended-precision reference
 (tests/xref.py, bound of tests/posterior_checks.py) on the constructed layouts of tests/layouts.py: every state the
 reference's `probability` can be in, on each code path of the update (two-pass kernels, 64-bit entry words, the tile
-layout, the host packer, the eight-lane model-1 row pass), the -G restriction, weighted files, row shards on one GPU and
+layout, the host packer), the -G restriction, weighted files, row shards on one GPU and
 under torchrun, the export, and full-size problems against the float64 oracle.  Each check prints one ELEMENTWISE line
 under `pytest -s`."""
 import os
@@ -201,27 +201,6 @@ def test_gpu_posterior_row_shards_on_one_gpu(R):
             assert np.array_equal(got.view(np.uint64), want[h].view(np.uint64)), (model, h)
         pc.check(pc.entry_values(want, ip, ix, x), x.e_step(theta[:, : d.H].T.cpu().numpy(), model),
                  pc.rtol_posterior(x, model), f"R={R} model {model}")
-
-
-M1_FIXED_WORKER = r'''
-import os, sys
-sys.path.insert(0, os.environ["GBRS_ROOT"])
-from tests.test_posterior_gpu import factory, problem, states
-for H in range(1, 9):
-    d, gene_of, x, eff = problem(H)
-    states(H, "GBRS_M1_FIXED", factory(d), d, x, eff)
-print("M1-FIXED-OK")
-'''
-
-
-def test_gpu_posterior_model1_eight_lane_row_pass(tmp_path):
-    """GBRS_M1_FIXED (read once per process, so in a process of its own)."""
-    script = tmp_path / "worker.py"
-    script.write_text(M1_FIXED_WORKER)
-    env = dict(os.environ, GBRS_ROOT=ROOT, GBRS_M1_FIXED="1")
-    res = subprocess.run([sys.executable, str(script)], env=env, capture_output=True, text=True, timeout=900)
-    print("\n".join(line for line in res.stdout.splitlines() if "model 1" in line))
-    assert res.returncode == 0 and "M1-FIXED-OK" in res.stdout, res.stdout[-2000:] + res.stderr[-3000:]
 
 
 def full_size_check(d, model, updates):

@@ -142,51 +142,3 @@ def test_config4_diploid_matches_oracle_on_a_2m_class_slice():
     out = gpu_fixed(d, 4, 8, gtmask=gm)
     assert_parity(out, o, 8, d, 4)
     assert np.all(out["counts"][gm == 0] == 0.0)
-
-
-M1_FIXED_WORKER = r'''
-import os, sys
-sys.path.insert(0, os.environ["GBRS_ROOT"])
-import numpy as np
-from gbrs_b200 import synth
-from gbrs_b200.emfactory import EMfactory
-from tests import helpers as hp
-for name in ("em_small_m1", "em_small_m1_diploid"):
-    g = hp.load_golden(name)
-    d = hp.synth_from_golden(g)
-    apm = synth.to_apm(d)
-    if g["masked"]:
-        apm.multiply(g["gtmask"], axis=2)
-        apm.eliminate_zeros()
-    em = EMfactory(apm)
-    em.target_lengths = synth.effective_lengths(d)
-    em.prepare(pseudocount=g["pseudocount"])
-    em.run(model=1, tol=g["tol"], max_iters=g["max_iters"], verbose=False)
-    assert em.num_iters == g["iters"], (em.num_iters, g["iters"])
-    assert hp.relerr(em.expected_read_counts(), g["counts"]) < 1e-9
-d = synth.generate(T=1500, N=40000, H=8, sample_index=5, wide_frac=0.02)
-o = hp.oracle_run(d, 1)
-em = EMfactory(synth.to_apm(d))
-em.target_lengths = synth.effective_lengths(d)
-em.prepare()
-em.run(model=1, tol=1e-4, max_iters=999, verbose=False)
-assert em.num_iters == o["iters"] and hp.relerr(em.expected_read_counts(), o["counts"]) < 1e-9
-print("M1-FIXED-OK")
-'''
-
-
-@pytest.mark.gpu
-def test_gpu_model1_eight_lane_row_pass_opt_in(tmp_path):
-    """GBRS_M1_FIXED (the opt-in model-1 row pass, read once per process): reference goldens and a medium problem with
-    wide classes against the oracle, in a process of its own.  Verified on the CPU through the SIMT shim
-    (tests/test_em_simt.py); first device run pending at the end of round 1."""
-    import os
-    import subprocess
-    import sys
-
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = tmp_path / "worker.py"
-    script.write_text(M1_FIXED_WORKER)
-    env = dict(os.environ, GBRS_ROOT=root, GBRS_M1_FIXED="1")
-    res = subprocess.run([sys.executable, str(script)], env=env, capture_output=True, text=True, timeout=900)
-    assert res.returncode == 0 and "M1-FIXED-OK" in res.stdout, res.stdout[-2000:] + res.stderr[-3000:]

@@ -52,15 +52,14 @@ timeout 900 compute-sanitizer --tool racecheck --error-exitcode 9 python -m pyte
   -k "golden" > $out/${tag}_racecheck_reconstruct.log 2>&1; echo "racecheck reconstruct rc=$?"
 tail -3 $out/${tag}_racecheck_reconstruct.log
 
-echo "== model 1: generic row pass vs the opt-in eight-lanes-per-class row pass (GBRS_M1_FIXED)"
+echo "== model 1"
 timeout 900 python bench.py --model 1 --steps 20 --warmup 3 --no-cpu > $out/${tag}_bench_c2_model1.json 2> $out/${tag}_bench_c2_model1.err; echo "m1 rc=$?"
-GBRS_M1_FIXED=1 timeout 900 python bench.py --model 1 --steps 20 --warmup 3 --no-cpu > $out/${tag}_bench_c2_model1_fixed.json 2> $out/${tag}_bench_c2_model1_fixed.err; echo "m1 fixed rc=$?"
 python - <<PY
 import json
-for n in ("${tag}_bench_c2_model1", "${tag}_bench_c2_model1_fixed"):
-    try:
-        d = json.loads(open("$out/" + n + ".json").read().strip().splitlines()[-1])
-        print(n, "ms_per_step", d["ms_per_step"], "row_pass_ms", d["roofline"]["per_kernel_ms"]["row_pass"])
-    except Exception as e:
-        print(n, "unreadable:", e)
+n = "${tag}_bench_c2_model1"
+try:
+    d = json.loads(open("$out/" + n + ".json").read().strip().splitlines()[-1])
+    print(n, "ms_per_step", d["ms_per_step"], "row_pass_ms", d["roofline"]["per_kernel_ms"]["row_pass"])
+except Exception as e:
+    print(n, "unreadable:", e)
 PY
